@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this implementation
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # + a seeded sample of the last timed step's outputs
 
 Workload of the headline line (BASELINE.json configs[1]): 2-D bilinear interpolation of a
 4096x4096 float64 column-major grid at 1e8 scattered queries per GPU ("step" = one pass over
@@ -74,6 +75,20 @@ def measured_peak():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_SAMPLE = 1 << 22               # float64 outputs kept by --dump-outputs: 32 MiB of the 800 MB a step writes
+DUMP_SEED = 2238
+
+
+def dump_outputs(out_dir, torch, zq):
+    """Write a fixed, seeded sample of the headline step's outputs to out_dir/interp2_scattered_zq.npy (float64),
+    so that two builds run with the same arguments can be compared output for output.  The sample is the
+    outputs at the sorted unique indices of DUMP_SAMPLE draws from default_rng(DUMP_SEED).integers(0, NQ)."""
+    idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, zq.numel(), DUMP_SAMPLE))
+    sample = zq[torch.from_numpy(idx).to(zq.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "interp2_scattered_zq.npy"), sample)
 
 
 def make_grid():
@@ -249,6 +264,8 @@ def main():
     ap.add_argument("--config5-full", action="store_true", help="(default now) profile-map stability at R = 1000 (1e6 neurons per column)")
     ap.add_argument("--no-config5-full", action="store_true", help="skip the R = 1000 profile-map stability")
     ap.add_argument("--only-config5", action="store_true", help="of the secondary workloads run only the profile-map stability")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write a seeded sample of the last step's outputs (rank 0) to DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)      # both arms: at least 3 warm-up steps
     if args.impl == "reference":
@@ -298,6 +315,8 @@ def main():
     ms = time_steps(torch, step, args.steps, 0, dist)
     gpu_launches = int(L_.lib().b200_launch_count() - launches0)   # counted by the library at every launch site
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, zq)      # now: the secondary workloads below reuse zq
     ms_per_step = ms / args.steps
     value = n_gpus * NQ / (ms_per_step * 1e-3)
     peak, peak_src = measured_peak()
@@ -597,7 +616,7 @@ def main():
                     m.close()
                 if rank == 0 and n_gpus == 1 and not args.no_cpu:
                     # the baseline beside it: the UNMODIFIED reference (oracle/_ref: its own FP32 kernels, compiled for
-                    # sm_100a where /root/reference exists) timed on this GPU — a baseline leg, never the thing shipped
+                    # sm_100a where B200_REFERENCE_DIR names it at build time) timed on this GPU — a baseline leg, never the thing shipped
                     # (in a child process: the reference's error convention is exit(-1), EventDrivenMap.cu:18-54)
                     try:
                         import re, subprocess

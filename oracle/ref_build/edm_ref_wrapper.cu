@@ -2,7 +2,7 @@
  * oracle/_ref/libedm_ref.so.  TEST INFRASTRUCTURE ONLY (the pin for oracle/ and for the product's
  * FP32 compatibility mode); never linked, imported or called by the product.
  *
- * The reference translation unit is included where it lies (REF_DIR is -I/root/reference); nothing
+ * The reference translation unit is included where it lies (-I$(REF), the reference checkout); nothing
  * of it is copied into this repository.  `private` is lifted so that the device buffers the
  * reference's own Save* dumpers print with "%f" (EventDrivenMap.cu:406-503) can be read back in
  * full precision instead.

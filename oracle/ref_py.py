@@ -17,9 +17,12 @@ M = 3  # noSpikes, parameters.hpp:12 (compile-time in the reference)
 
 
 def build():
-    """Compile the reference where it lies (only possible where /root/reference exists)."""
-    if os.path.isdir("/root/reference"):
-        subprocess.check_call(["make", "-C", os.path.join(_HERE, "ref_build")], stdout=subprocess.DEVNULL)
+    """Compile the reference where it lies: the checkout of the reference project that the environment
+    variable B200_REFERENCE_DIR names (the reference is not part of this repository; without it, nothing)."""
+    ref_dir = os.environ.get("B200_REFERENCE_DIR")
+    if ref_dir and os.path.isdir(ref_dir):
+        subprocess.check_call(["make", "-C", os.path.join(_HERE, "ref_build"), "REF=" + os.path.abspath(ref_dir)],
+                              stdout=subprocess.DEVNULL)
     return os.path.exists(REF_SO)
 
 

@@ -130,7 +130,7 @@ def test_product_against_the_reference_live(b200, oracle):
     same front cells as the product's FP32 mode and the FP32 oracle, F to FP32 noise."""
     from oracle import ref_py
     if not ref_py.available():
-        pytest.skip("oracle/_ref was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref was not built (needs B200_REFERENCE_DIR at build time)")
     rng = np.random.default_rng(5)
     for k in range(4):
         z = GUESS * (1 + 0.03 * rng.standard_normal(3))

@@ -1,4 +1,4 @@
-import sys; sys.path.insert(0, '/root/repo')
+import os, sys; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import armadillocudalinearinterpolation_b200 as B, bench
 for prec in ("f64", "f32"):

@@ -1,6 +1,6 @@
 """Headline kernel with linspace (affine), B200_INTERP_AFFINE=0 (shared-memory tables) and non-uniform axes."""
 import os, sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import armadillocudalinearinterpolation_b200 as B
 n = 4096

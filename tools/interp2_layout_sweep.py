@@ -1,6 +1,6 @@
 """Scattered interp2, 1e8 queries: column-major Z vs 2x2 corner records vs overlapping 4x4 tiles, by grid size."""
-import sys
-sys.path.insert(0, "/root/repo")
+import os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import armadillocudalinearinterpolation_b200 as B
 P = B.Interp2Plan

@@ -1,5 +1,5 @@
 import os, sys, time
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import armadillocudalinearinterpolation_b200 as B
 import bench

@@ -1,6 +1,6 @@
 """ncu driver for the kernels outside prof_driver.py: the opt-in banded pipeline and the interp1 shared-memory path."""
-import sys
-sys.path.insert(0, "/root/repo")
+import os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import armadillocudalinearinterpolation_b200 as B
 import bench

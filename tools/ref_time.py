@@ -7,7 +7,7 @@ import numpy as np
 from oracle import ref_py
 import bench
 if not ref_py.available():
-    sys.exit("oracle/_ref/libedm_ref.so is missing (built where /root/reference exists)")
+    sys.exit("oracle/_ref/libedm_ref.so is missing (built where B200_REFERENCE_DIR names the reference)")
 z0 = np.array(bench.Z_DRIVER, np.float64)
 for N in (1024, 512):
     ms = ref_py.time_compute_f(z0, bench.BETA, 1000, N=N, warm=3, reps=10)
