@@ -672,11 +672,7 @@ edm_evolve_kernel(const EvolveArgs<T> A) {
   };
 
   constexpr bool kStraight = (MINB <= 4);
-#ifdef B200_EDM_CAPPED_STRAIGHT   // experiment hook: the stage-wise scan (4 neurons at a time) on the capped build — 3.61 vs 3.31 ms, not taken
-  auto scan = [&](int parity) { scan_straight(parity); };
-#else
   auto scan = [&](int parity) { if (kStraight) scan_straight(parity); else scan_branchy(parity); };
-#endif
 
   // The event message: (dt, idx) and the event-uniform advance coefficients.
   const bool prof = A.profile_nc != 0;
@@ -1437,40 +1433,23 @@ int ensure_u(b200_edm* g, size_t n) {
 
 // every device holds `slot_bytes` of results at slot d of its gather buffer: exchange them so that every
 // device (in particular the primary) holds all slots.  One in-place ncclAllGather per device inside one
-// group (single process driving several devices); without communicators (B200_EDM_NO_NCCL=1) the
-// helpers' slots are peer-copied to the primary instead.
+// group (single process driving several devices; b200_edm_set_devices created the communicators).
 int exchange_slots(b200_edm* h, cudaStream_t st, size_t slot_bytes, size_t acc_slot_items) {
   const size_t ndev = h->helpers.size() + 1;
-  if (!h->comms.empty()) {
-    NvtxRange nvtx("edm:nccl_all_gather");
-    B200_NCCL(g_nccl.group_start());
-    ncclResult_t bad = ncclSuccess;   // a failed call must not leave the thread inside an open group
-    for (size_t d = 0; d < ndev && bad == ncclSuccess; ++d) {
-      b200_edm* g = dev_handle(h, d);
-      cudaStream_t gs = d == 0 ? st : g->stream;
-      if (slot_bytes)
-        bad = g_nccl.all_gather((const char*)g->d_gather + d * slot_bytes, g->d_gather, slot_bytes, ncclChar, h->comms[d], gs);
-      if (acc_slot_items && bad == ncclSuccess)
-        bad = g_nccl.all_gather(g->d_gather_acc + d * acc_slot_items, g->d_gather_acc, acc_slot_items, ncclInt32, h->comms[d], gs);
-    }
-    const ncclResult_t end = g_nccl.group_end();
-    if (bad != ncclSuccess) return fail(B200_ERR_CUDA, "NCCL error %d (%s) in ncclAllGather", (int)bad, g_nccl.error_string(bad));
-    if (end != ncclSuccess) return fail(B200_ERR_CUDA, "NCCL error %d (%s) in ncclGroupEnd", (int)end, g_nccl.error_string(end));
-    return B200_OK;
-  }
-  for (size_t d = 1; d < ndev; ++d) {
+  NvtxRange nvtx("edm:nccl_all_gather");
+  B200_NCCL(g_nccl.group_start());
+  ncclResult_t bad = ncclSuccess;   // a failed call must not leave the thread inside an open group
+  for (size_t d = 0; d < ndev && bad == ncclSuccess; ++d) {
     b200_edm* g = dev_handle(h, d);
-    B200_CUDA(cudaSetDevice(g->device));
+    cudaStream_t gs = d == 0 ? st : g->stream;
     if (slot_bytes)
-      B200_CUDA(cudaMemcpyPeerAsync((char*)h->d_gather + d * slot_bytes, h->device, (const char*)g->d_gather + d * slot_bytes,
-                                    g->device, slot_bytes, g->stream));
-    if (acc_slot_items)
-      B200_CUDA(cudaMemcpyPeerAsync(h->d_gather_acc + d * acc_slot_items, h->device, g->d_gather_acc + d * acc_slot_items,
-                                    g->device, acc_slot_items * sizeof(int32_t), g->stream));
-    B200_CUDA(cudaEventRecord(g->ev_done, g->stream));
+      bad = g_nccl.all_gather((const char*)g->d_gather + d * slot_bytes, g->d_gather, slot_bytes, ncclChar, h->comms[d], gs);
+    if (acc_slot_items && bad == ncclSuccess)
+      bad = g_nccl.all_gather(g->d_gather_acc + d * acc_slot_items, g->d_gather_acc, acc_slot_items, ncclInt32, h->comms[d], gs);
   }
-  B200_CUDA(cudaSetDevice(h->device));
-  for (size_t d = 1; d < ndev; ++d) B200_CUDA(cudaStreamWaitEvent(st, h->helpers[d - 1]->ev_done, 0));
+  const ncclResult_t end = g_nccl.group_end();
+  if (bad != ncclSuccess) return fail(B200_ERR_CUDA, "NCCL error %d (%s) in ncclAllGather", (int)bad, g_nccl.error_string(bad));
+  if (end != ncclSuccess) return fail(B200_ERR_CUDA, "NCCL error %d (%s) in ncclGroupEnd", (int)end, g_nccl.error_string(end));
   return B200_OK;
 }
 
@@ -1782,10 +1761,8 @@ int b200_edm_set_devices(b200_edm* h, const int* device_ids, size_t ndevices) {
     }
   }
   cudaSetDevice(h->device);
-  // the exchange is one NCCL all-gather per evaluation batch (north-star; SURVEY 8e); B200_EDM_NO_NCCL=1 keeps
-  // the round-1 peer-copy exchange for A/B timing
-  const char* no_nccl = getenv("B200_EDM_NO_NCCL");
-  if (rc == B200_OK && ndevices > 1 && !(no_nccl && no_nccl[0] == '1')) {
+  // the exchange is one NCCL all-gather per evaluation batch (north-star; SURVEY 8e)
+  if (rc == B200_OK && ndevices > 1) {
     if (!load_nccl()) rc = fail(B200_ERR_UNSUPPORTED, "edm_set_devices: libnccl.so.2 could not be loaded (%s)", dlerror());
     if (rc == B200_OK) {
       h->comms.resize(ndevices);

@@ -88,10 +88,9 @@ struct StagePool {
 template <class Launch>
 int staged_run(StagePool& pool, int device, const std::vector<StageArray>& arrays, size_t n, Launch launch) {
   if (n == 0) return B200_OK;
-  static const size_t kChunkElems = [] { const char* e = getenv("B200_STAGE_CHUNK_LOG2"); const int v = e ? atoi(e) : 0; return (size_t)1 << ((v >= 12 && v <= 24) ? v : 20); }();
+  constexpr size_t kChunkElems = (size_t)1 << 20;
   unsigned hw = std::thread::hardware_concurrency();
   int nworkers = (int)(hw >= 16 ? 8 : (hw >= 4 ? hw / 2 : 1));
-  { const char* e = getenv("B200_STAGE_THREADS"); const int v = e ? atoi(e) : 0; if (v >= 1 && v <= 64) nworkers = v; }
   const size_t nchunks = (n + kChunkElems - 1) / kChunkElems;
   if ((size_t)nworkers > nchunks) nworkers = (int)nchunks;
   B200_TRY(pool.ensure(device, nworkers, kChunkElems, arrays));

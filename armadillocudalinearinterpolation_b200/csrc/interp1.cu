@@ -20,7 +20,6 @@
 //             binary search only inside pathological buckets;
 //  * the blend is (1-w)*Y[a] + w*Y[b] with w = |X[a]-q| / (|X[a]-q| + |X[b]-q|), every
 //    operation individually rounded (__dmul_rn, ...), bit-identical to the CPU oracle.
-#include <cstdlib>
 #include "interp_common.cuh"
 #include "host_staging.cuh"
 
@@ -32,62 +31,15 @@ template <typename T> struct Loader1;
 template <> struct Loader1<double> { using type = LoadSeg1D; };
 template <> struct Loader1<float> { using type = LoadSeg1F; };
 
-// ---- non-uniform knots: one record per uniform bin (round 2; opt-in, see plan1_create for the measurement) ----
-// The general path costs two DEPENDENT gathers per query (first2[bin], then the segment record, then more
-// records while scanning forward).  A bin record holds everything a query of that bin normally needs in ONE
-// line: a0 = the last knot before the bin, the number of knots inside the bin, and knots / values a0, a0+1, a0+2
-// (clamped at the last knot).  A query resolves from the record alone unless its bracket starts at a0+2 or later
-// (bins holding >= 2 knots below the query), in which case it continues with the segment records as before.
-// 64 bytes per bin for double, 32 for float; the bracket is still fixed by comparing against stored knots.
 template <typename T>
-struct alignas(sizeof(T) == 8 ? 64 : 32) BinRec {
-  int32_t a0, cnt;
-  T x[3], y[3];
-};
-
-template <typename T>
-__global__ void build_binrec_kernel(const T* __restrict__ x, const T* __restrict__ y, const int32_t* __restrict__ first,
-                                    int n, int nb, BinRec<T>* __restrict__ rec) {
-  const int k = blockIdx.x * blockDim.x + threadIdx.x;
-  if (k >= nb) return;
-  BinRec<T> r;
-  r.a0 = max(first[k] - 1, 0);
-  r.cnt = first[k + 1] - first[k];
-#pragma unroll
-  for (int i = 0; i < 3; ++i) { const int j = min(r.a0 + i, n - 1); r.x[i] = x[j]; r.y[i] = y[j]; }
-  rec[k] = r;
-}
-
-__device__ __forceinline__ BinRec<double> ld_binrec(const BinRec<double>* p) {
-  double a[4], b[4];
-  ld_keep_256(reinterpret_cast<const double*>(p), a);
-  ld_keep_256(reinterpret_cast<const double*>(p) + 4, b);
-  BinRec<double> r;
-  const long long bits = __double_as_longlong(a[0]);
-  r.a0 = (int32_t)(bits & 0xffffffffll); r.cnt = (int32_t)(bits >> 32);
-  r.x[0] = a[1]; r.x[1] = a[2]; r.x[2] = a[3]; r.y[0] = b[0]; r.y[1] = b[1]; r.y[2] = b[2];
-  return r;
-}
-__device__ __forceinline__ BinRec<float> ld_binrec(const BinRec<float>* p) {
-  float a[4], b[4];
-  const uint64_t pol = l2_policy_evict_last();
-  ld_keep_128(reinterpret_cast<const float*>(p), a, pol);
-  ld_keep_128(reinterpret_cast<const float*>(p) + 4, b, pol);
-  BinRec<float> r;
-  r.a0 = __float_as_int(a[0]); r.cnt = __float_as_int(a[1]);
-  r.x[0] = a[2]; r.x[1] = a[3]; r.x[2] = b[0]; r.y[0] = b[1]; r.y[1] = b[2]; r.y[2] = b[3];
-  return r;
-}
-
-template <typename T>
-__device__ __forceinline__ T interp1_one(const AxisDev<T>& ax, const typename Loader1<T>::type& ld,
-                                         const BinRec<T>* __restrict__ rec, T q, T extrap, int32_t& idx) {
+__device__ __forceinline__ T interp1_one(const AxisDev<T>& ax, const typename Loader1<T>::type& ld, T q, T extrap,
+                                         int32_t& idx) {
   if (!(q >= ax.x0 && q <= ax.xmax)) {  // out of range -> extrap_val; NaN query -> NaN
     idx = -1;
     return (q != q) ? qnan<T>() : extrap;
   }
   Seg1<T> sg;
-  if (sizeof(T) == 8 && ax.mode == 0 && !rec) {
+  if (sizeof(T) == 8 && ax.mode == 0) {
     // (quasi-)uniform knots, double: the common case — the arithmetic bin is the bracket, the weight operands are in
     // the normal range — as straight-line code with the branch-free divide; anything else takes the generic walk
     const int k = bin_of(ax, q);
@@ -99,25 +51,7 @@ __device__ __forceinline__ T interp1_one(const AxisDev<T>& ax, const typename Lo
       return blend((T)div_rn_fast(a_err, sum), sg.ya, sg.yb);
     }
   }
-  if (rec) {
-    const BinRec<T> r = ld_binrec(rec + bin_of(ax, q));
-    const bool up1 = (r.a0 + 1 < ax.n) && (r.x[1] <= q);
-    const bool up2 = (r.a0 + 2 < ax.n) && (r.x[2] <= q);
-    if (!up2) {   // the bracket is a0 or a0 + 1: everything is in the record
-      idx = r.a0 + (up1 ? 1 : 0);
-      sg.xa = up1 ? r.x[1] : r.x[0]; sg.xb = up1 ? r.x[2] : r.x[1];
-      sg.ya = up1 ? r.y[1] : r.y[0]; sg.yb = up1 ? r.y[2] : r.y[1];
-    } else if (r.cnt > kLinearScanMax) {
-      idx = find_bracket(ax, ld, q, sg);   // clustered knots: the bounded binary search of the table path
-    } else {
-      int a = r.a0 + 2;
-      sg = ld(a);
-      while (sg.xb <= q && a + 1 < ax.n) { a += 1; sg = ld(a); }
-      idx = a;
-    }
-  } else {
-    idx = find_bracket(ax, ld, q, sg);
-  }
+  idx = find_bracket(ax, ld, q, sg);
   return blend(weight_of(sg.xa, sg.xb, q), sg.ya, sg.yb);
 }
 
@@ -132,8 +66,8 @@ template <> __device__ __forceinline__ LoadSeg1F make_loader1<float>(const float
 // of this kernel at 1e7 and 1e8 queries — the gather RATE bounds it, not the bytes — and not kept.)
 template <typename T, bool WANT_IDX>
 __global__ void __launch_bounds__(kThreads)
-interp1_vec_kernel(AxisDev<T> ax, const T* __restrict__ seg, const BinRec<T>* __restrict__ rec,
-                   const T* __restrict__ xi, T* __restrict__ yi, int32_t* __restrict__ idx, size_t nvec, T extrap) {
+interp1_vec_kernel(AxisDev<T> ax, const T* __restrict__ seg, const T* __restrict__ xi, T* __restrict__ yi,
+                   int32_t* __restrict__ idx, size_t nvec, T extrap) {
   constexpr int V = Vec256<T>::n;
   // programmatic dependent launch (plan1_launch): this grid may have been scheduled while the previous kernel of
   // the stream was still draining; nothing is read or written before that kernel has completed and flushed
@@ -147,7 +81,7 @@ interp1_vec_kernel(AxisDev<T> ax, const T* __restrict__ seg, const BinRec<T>* __
     int32_t id[V];
     ld_stream_256(xi + i * V, q);
 #pragma unroll
-    for (int j = 0; j < V; ++j) y[j] = interp1_one<T>(ax, ld, rec, q[j], extrap, id[j]);
+    for (int j = 0; j < V; ++j) y[j] = interp1_one<T>(ax, ld, q[j], extrap, id[j]);
     st_stream_256(yi + i * V, y);
     if (WANT_IDX) {
       if (V == 8) {
@@ -162,14 +96,13 @@ interp1_vec_kernel(AxisDev<T> ax, const T* __restrict__ seg, const BinRec<T>* __
 // Scalar kernel: tails and unaligned buffers.
 template <typename T, bool WANT_IDX>
 __global__ void __launch_bounds__(kThreads)
-interp1_scalar_kernel(AxisDev<T> ax, const T* __restrict__ seg, const BinRec<T>* __restrict__ rec,
-                      const T* __restrict__ xi, T* __restrict__ yi, int32_t* __restrict__ idx, size_t begin,
-                      size_t end, T extrap) {
+interp1_scalar_kernel(AxisDev<T> ax, const T* __restrict__ seg, const T* __restrict__ xi, T* __restrict__ yi,
+                      int32_t* __restrict__ idx, size_t begin, size_t end, T extrap) {
   const auto ld = make_loader1<T>(seg);
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = begin + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < end; i += stride) {
     int32_t id;
-    yi[i] = interp1_one<T>(ax, ld, rec, xi[i], extrap, id);
+    yi[i] = interp1_one<T>(ax, ld, xi[i], extrap, id);
     if (WANT_IDX) idx[i] = id;
   }
 }
@@ -249,7 +182,6 @@ struct b200_interp1_plan {
   Axis<float> ax32;
   void* yg = nullptr;   // device copy of the values
   void* seg = nullptr;  // [ng][4] segment records
-  void* binrec = nullptr;  // [nb] bin records (non-uniform knots), or nullptr
   size_t smem_bytes = 0;  // > 0: the grid fits the shared-memory path
   cudaStream_t stream[2] = {nullptr, nullptr};
   // staging for host-buffer execution (allocated on first use)
@@ -272,11 +204,6 @@ int plan1_build_seg(b200_interp1_plan* p, cudaStream_t st) {
   Axis<T>& A = axis_of<T>(p);
   build_seg1_kernel<T><<<grid_for(p->ng), kThreads, 0, B200_CNT(st)>>>(A.x, (const T*)p->yg, (int)p->ng,
                                                              (T*)p->seg);
-  if (p->binrec) {
-    const AxisDev<T>& d = A.dev;
-    build_binrec_kernel<T><<<grid_for((size_t)d.nb), kThreads, 0, B200_CNT(st)>>>(A.x, (const T*)p->yg, d.first, d.n, d.nb,
-                                                                                (BinRec<T>*)p->binrec);
-  }
   B200_CUDA(cudaGetLastError());
   return B200_OK;
 }
@@ -292,16 +219,6 @@ int plan1_create(b200_interp1_plan* p, const T* xg, const T* yg, size_t ng) {
   B200_CUDA(cudaMemsetAsync(p->yg, 0, ng * sizeof(T) + 16, p->stream[0]));
   B200_CUDA(cudaMalloc(&p->seg, ng * 4 * sizeof(T)));
   B200_CUDA(cudaMemcpyAsync(p->yg, yg, ng * sizeof(T), cudaMemcpyHostToDevice, p->stream[0]));
-  {
-    // bin records for non-uniform knots: OPT-IN (B200_INTERP1_BINREC=1).  Measured at 1e6 knots x 1e7 queries
-    // (tools/interp1_cfg1_sweep.py): unsorted 110 -> 101 us, sorted 53 -> 56 us — a random gather costs one LSU
-    // wavefront per lane per load instruction, so one 64-byte record (two 256-bit loads) is no cheaper than the
-    // 8-byte bucket entry + 32-byte segment record it replaces, and the table doubles (64 MB).
-    const AxisDev<T>& d = axis_of<T>(p).dev;
-    const char* e = getenv("B200_INTERP1_BINREC");
-    if (d.mode == 1 && (size_t)d.nb * sizeof(BinRec<T>) <= ((size_t)96 << 20) && (e && e[0] == '1'))
-      B200_CUDA(cudaMalloc(&p->binrec, (size_t)d.nb * sizeof(BinRec<T>)));
-  }
   B200_TRY(plan1_build_seg<T>(p, p->stream[0]));
   B200_CUDA(cudaStreamSynchronize(p->stream[0]));
   {
@@ -309,8 +226,7 @@ int plan1_create(b200_interp1_plan* p, const T* xg, const T* yg, size_t ng) {
     const AxisDev<T>& ax = axis_of<T>(p).dev;
     const size_t need = 16 + (ax.affine ? 1 : 2) * pad16(sizeof(T) * ng) +
                         ((!ax.affine && ax.mode) ? pad16(sizeof(int32_t) * ((size_t)ax.nb + 1)) : 0);
-    const char* e = getenv("B200_INTERP1_SMEM");
-    p->smem_bytes = (need <= 100 * 1024 && !(e && e[0] == '0')) ? need : 0;   // two CTAs per SM
+    p->smem_bytes = need <= 100 * 1024 ? need : 0;   // two CTAs per SM
   }
   return B200_OK;
 }
@@ -328,14 +244,9 @@ int plan1_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* i
   size_t nvec = aligned ? ni / V : 0;
   if (nvec && p->smem_bytes && nvec >= 4096) {
     auto launch = [&](auto kern) -> int {
-      B200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem_bytes));
-      int per_sm = 1, sms = 148;
-      B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kSmem1Threads, p->smem_bytes));
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device);
-      const size_t blocks = (nvec + kSmem1Threads - 1) / kSmem1Threads;
-      const size_t resident = (size_t)sms * (per_sm > 0 ? per_sm : 1);
-      kern<<<(int)(blocks < resident ? blocks : resident), kSmem1Threads, p->smem_bytes, B200_CNT(st)>>>(
-          ax, (const T*)p->yg, xi, yi, idx, nvec, extrap);
+      unsigned grid = 0;
+      B200_TRY(persistent_grid(kern, kSmem1Threads, p->smem_bytes, p->device, (nvec + kSmem1Threads - 1) / kSmem1Threads, grid));
+      kern<<<grid, kSmem1Threads, p->smem_bytes, B200_CNT(st)>>>(ax, (const T*)p->yg, xi, yi, idx, nvec, extrap);
       return B200_OK;
     };
     if (idx) B200_TRY(launch(interp1_smem_kernel<T, true>));
@@ -344,32 +255,28 @@ int plan1_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* i
     // a few waves of 8 resident CTAs per SM, grid-stride beyond that
     size_t blocks = (nvec + kThreads - 1) / kThreads;
     // measured: 1e7 queries 37.0 us with 16 CTAs per SM vs 38.9 us with 64; 1e8 queries 0.304 ms with 64 vs 0.316 ms with 16
-    static const size_t forced = [] { const char* e = getenv("B200_INTERP1_GRID_MULT"); return (size_t)(e && atoi(e) > 0 ? atoi(e) : 0); }();
-    const size_t mult = forced ? forced : (blocks > (size_t)148 * 256 ? 64 : 16);
+    const size_t mult = blocks > (size_t)148 * 256 ? 64 : 16;
     int grid = (int)(blocks < (size_t)148 * mult ? blocks : (size_t)148 * mult);
-    const BinRec<T>* rec = (const BinRec<T>*)p->binrec;
     // back-to-back calls on one stream (a caller that batches, the chunks of the host-buffer pipeline): with the
     // programmatic-stream-serialization attribute the next grid is scheduled while this one drains and starts the
-    // moment it has completed — no launch bubble between 30-60 us kernels.  B200_INTERP1_PDL=0: ordinary launches.
-    static const bool pdl = [] { const char* e = getenv("B200_INTERP1_PDL"); return !(e && atoi(e) == 0); }();
+    // moment it has completed — no launch bubble between 30-60 us kernels
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = 0; cfg.stream = B200_CNT(st);
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
+    cfg.attrs = attr; cfg.numAttrs = 1;
     int32_t* no_idx = nullptr;
-    if (idx) B200_CUDA(cudaLaunchKernelEx(&cfg, interp1_vec_kernel<T, true>, ax, seg, rec, xi, yi, idx, nvec, extrap));
-    else B200_CUDA(cudaLaunchKernelEx(&cfg, interp1_vec_kernel<T, false>, ax, seg, rec, xi, yi, no_idx, nvec, extrap));
+    if (idx) B200_CUDA(cudaLaunchKernelEx(&cfg, interp1_vec_kernel<T, true>, ax, seg, xi, yi, idx, nvec, extrap));
+    else B200_CUDA(cudaLaunchKernelEx(&cfg, interp1_vec_kernel<T, false>, ax, seg, xi, yi, no_idx, nvec, extrap));
   }
   size_t done = nvec * V;
   if (done < ni) {
     size_t rem = ni - done;
     size_t blocks = (rem + kThreads - 1) / kThreads;
     int grid = (int)(blocks < (size_t)148 * 64 ? blocks : (size_t)148 * 64);
-    const BinRec<T>* rec = (const BinRec<T>*)p->binrec;
-    if (idx) interp1_scalar_kernel<T, true><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, rec, xi, yi, idx, done, ni, extrap);
-    else interp1_scalar_kernel<T, false><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, rec, xi, yi, nullptr, done, ni, extrap);
+    if (idx) interp1_scalar_kernel<T, true><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, idx, done, ni, extrap);
+    else interp1_scalar_kernel<T, false><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, nullptr, done, ni, extrap);
   }
   B200_CUDA(cudaGetLastError());
   return B200_OK;
@@ -436,7 +343,6 @@ void plan1_free(b200_interp1_plan* p) {
   p->ax32.release();
   cudaFree(p->yg);
   cudaFree(p->seg);
-  cudaFree(p->binrec);
   for (int s = 0; s < 2; ++s) {
     cudaFree(p->st_in[s]); cudaFree(p->st_out[s]); cudaFree(p->st_idx[s]);
     if (p->stream[s]) cudaStreamDestroy(p->stream[s]);

@@ -26,6 +26,7 @@ constexpr int kBandThreads = 512;   // 4 consecutive queries per thread and roun
 constexpr int kBandQ = 4;
 constexpr int kBandRound = kBandThreads * kBandQ;   // 2048 queries per round; a chunk is 1 or 2 rounds
 constexpr int kBandMaxK = 64;
+constexpr size_t kBandBytes = (size_t)32 << 20;   // records per band (sweep: 64 MiB 2.52, 32 MiB 2.27, 16 MiB 2.27, 8 MiB 2.75 ms; profiles/interp2_banded_r1.md)
 
 struct BandDev {
   int shift;          // band = ax >> shift

@@ -48,7 +48,7 @@ void NewtonSolver::Solve(arma::vec& solution, arma::vec& residualHistory, ExitFl
   // turns out to be converged is then computed in vain).  `jacobian` stays the last Jacobian a step was taken with,
   // as in the reference (pJacobianExternal below).
   AbstractNonlinearProblemFused* fused = NULL;
-  if (mFuse && mpProblemJacobian && !std::getenv("B200_NEWTON_NO_FUSE") &&
+  if (mFuse && mpProblemJacobian &&
       dynamic_cast<void*>(mpProblem) == dynamic_cast<void*>(mpProblemJacobian))
     fused = dynamic_cast<AbstractNonlinearProblemFused*>(mpProblemJacobian);
   const bool oneBatch = fused && fused->PrefersOneBatchPerIterate();

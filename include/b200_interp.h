@@ -88,18 +88,19 @@ int b200_interp2_plan_create(b200_dtype dtype, const void* x, size_t nx, const v
  * B200_INTERP2_NO_CELLS keeps only the column-major matrix, B200_INTERP2_FORCE_CELLS always builds them. */
 #define B200_INTERP2_NO_CELLS 1u
 #define B200_INTERP2_FORCE_CELLS 2u
-/* Device-buffer scattered calls on a table too large for L2 first partition the queries by column
- * band of the records (<= 32 MiB per band) so that every record gather hits L2 (four streaming
- * passes instead of one 128-byte DRAM line fill per query; same bits).  B200_INTERP2_NO_BANDS
- * disables that path, B200_INTERP2_FORCE_BANDS takes it for every device-buffer call of a plan that
- * has corner records (tests).  Its scratch (26 B per query, f64) lives in the plan: as with the
- * grid call, one plan must not run on two streams at once. */
+/* Opt-in L2-banded pipeline: with B200_INTERP2_FORCE_BANDS the plan builds the corner records and every
+ * device-buffer scattered call first partitions the queries by column band of the records (<= 32 MiB
+ * per band) so that every record gather hits L2 (four streaming passes instead of one 128-byte DRAM line
+ * fill per query; same bits).  Grids too narrow for two bands, and plans with B200_INTERP2_NO_BANDS, take
+ * the direct kernels.  Its scratch (26 B per query, f64) lives in the plan: as with the grid call, one
+ * plan must not run on two streams at once. */
 #define B200_INTERP2_NO_BANDS 4u
 #define B200_INTERP2_FORCE_BANDS 8u
-/* Matrices of 112 MiB and more are additionally stored as overlapping 4x4 tiles (stride 3; 16/9 the
- * memory of Z): the four corners of any cell then sit in ONE 128-byte line of a table less than half
- * the size of the corner records, and scattered queries — bounded on B200 by DRAM row activations, one
- * per L2 miss — miss L2 correspondingly less often.  Same bits.  NO_TILES / FORCE_TILES override. */
+/* f64 matrices of more than 12 and less than 180 MiB are stored as overlapping 4x4 tiles (stride 3; 16/9
+ * the memory of Z) instead of corner records: the four corners of any cell then sit in ONE 128-byte line
+ * of a table less than half the size of the corner records, and scattered queries — bounded on B200 by
+ * DRAM row activations, one per L2 miss — miss L2 correspondingly less often.  Same bits.  NO_TILES /
+ * FORCE_TILES override; NO_CELLS / FORCE_CELLS without FORCE_TILES build no tiles. */
 #define B200_INTERP2_NO_TILES 16u
 #define B200_INTERP2_FORCE_TILES 32u
 /* Order of Armadillo's two separable passes.  Default: along X first (whole columns of Z blended into

@@ -151,38 +151,6 @@ def test_interp2_device_buffers(b200, oracle):
     assert same_bits(zi.cpu().numpy(), oracle.interp2_grid(x, y, z, xq[:100], yq[:64]))
 
 
-@pytest.mark.parametrize("dt", [np.float64, np.float32])
-@pytest.mark.parametrize("kind", ["cumsum", "clustered", "two_per_bin"])
-def test_interp1_bin_records_same_bits(b200, oracle, dt, kind, monkeypatch):
-    """Opt-in bin records for non-uniform knots (B200_INTERP1_BINREC=1: one 64-byte / 32-byte record per uniform
-    bin holding the three knots a query of that bin can need): same values and brackets as the oracle, including
-    bins with many knots (fall back to the segment records / binary search), the last knot and ragged tails."""
-    monkeypatch.setenv("B200_INTERP1_BINREC", "1")
-    rng = np.random.default_rng(31)
-    ng = 50_001
-    if kind == "cumsum":
-        xg = np.cumsum(0.5 + rng.random(ng))
-    elif kind == "clustered":
-        xg = np.concatenate([np.linspace(0, 1e-3, ng - 100), np.linspace(0.1, 1.0, 100)])
-    else:   # pairs of close knots: most bins hold two knots, the next pair is far
-        base = np.arange(ng // 2, dtype=np.float64) * 2.0
-        xg = np.sort(np.concatenate([base, base + 0.3 * rng.random(base.size) + 0.05]))
-        xg[ng // 4:] += 500.0          # and one large gap, so that the knots are not quasi-uniform
-    xg = np.unique(xg.astype(dt)); xg = ((xg - xg[0]) / (xg[-1] - xg[0])).astype(dt); xg = np.unique(xg)
-    yg = rng.standard_normal(xg.size).astype(dt)
-    xi = rng.uniform(-0.01, 1.01, 400_003).astype(dt)
-    xi[:5] = [xg[0], xg[-1], np.nan, xg[-2], np.nextafter(xg[-1], dt(2))]
-    xi[100:100 + 2000] = xg[::max(1, xg.size // 2000)][:2000]
-    plan = b200.Interp1Plan(xg, yg)
-    assert plan.lookup_mode == 1
-    yi, idx = plan(xi, extrap=-3.0, return_index=True)
-    yo, io = oracle.interp1(xg, yg, xi, extrap=-3.0, nthreads=8)
-    assert same_bits(yi, yo) and np.array_equal(idx, io)
-    yg2 = rng.standard_normal(xg.size).astype(dt)
-    plan.set_values(yg2)                                    # the records are rebuilt with the new values
-    assert same_bits(plan(xi, extrap=0.5), oracle.interp1(xg, yg2, xi, extrap=0.5, want_idx=False, nthreads=8))
-
-
 def _config1_inputs(kind):
     """BASELINE config 1 exactly as bench.py builds it (1e6 knots; SURVEY 8d seeds)."""
     ng = 1_000_000
@@ -358,19 +326,21 @@ def test_interp2_banded_pipeline_same_bits(b200, oracle, dt, shape):
     assert same_bits(out.cpu().numpy(), oracle.interp2_scattered(x, y, z, xq[1:], yq[1:], extrap=0.5, nthreads=8))
 
 
-def test_interp2_affine_axes_same_bits(b200, oracle, monkeypatch):
+def test_interp2_affine_axes_same_bits(b200, oracle):
     """linspace-style knots (x0 + j*step with two roundings, verified knot by knot at plan time) are
-    recomputed in the kernel instead of loaded; B200_INTERP_AFFINE=0 keeps the tables.  Same bits."""
+    recomputed in the kernel instead of loaded; with one knot of each axis moved by one ulp the axes are
+    not affine and the same queries take the tables.  Same bits."""
     rng = np.random.default_rng(19)
     x = np.linspace(-1.0, 2.0, 1500); y = np.linspace(0.0, 1.0, 700)
+    xp = x.copy(); xp[500] = np.nextafter(xp[500], 5.0)
+    yp = y.copy(); yp[300] = np.nextafter(yp[300], 5.0)
     z = rng.standard_normal((y.size, x.size))
     xq = rng.uniform(-1.1, 2.1, 400_003); yq = rng.uniform(-0.1, 1.1, 400_003)
     xq[:6] = [x[0], x[-1], np.nan, x[3], x[-2], np.nextafter(x[-1], 5.0)]; yq[:6] = [y[0], y[-1], 0.0, np.nan, y[-1], 0.5]
-    ref = oracle.interp2_scattered(x, y, z, xq, yq, extrap=-4.0, nthreads=8)
-    for affine in ("1", "0"):
-        monkeypatch.setenv("B200_INTERP_AFFINE", affine)
+    for kx, ky in ((x, y), (xp, yp)):
+        ref = oracle.interp2_scattered(kx, ky, z, xq, yq, extrap=-4.0, nthreads=8)
         for flags in (0, b200.Interp2Plan.FORCE_CELLS, b200.Interp2Plan.NO_CELLS):
-            assert same_bits(b200.Interp2Plan(x, y, z, flags=flags).scattered(xq, yq, extrap=-4.0), ref)
+            assert same_bits(b200.Interp2Plan(kx, ky, z, flags=flags).scattered(xq, yq, extrap=-4.0), ref)
 
 
 @pytest.mark.parametrize("dt", [np.float64, np.float32])
@@ -447,11 +417,10 @@ def test_interp2_fast_kernel_special_queries(b200, oracle, y_first):
 
 
 @pytest.mark.parametrize("y_first", [False, True])
-def test_interp2_locality_probe_both_kernels_same_bits(b200, oracle, y_first, monkeypatch):
+def test_interp2_locality_probe_both_kernels_same_bits(b200, oracle, y_first):
     """Large device-buffer batches on an affine/tile plan are served by one of two kernels, chosen on the device by a
-    locality probe (cell-sorted queries -> the straight-line kernel, random queries -> the generic one): both choices,
-    and the forced settings (B200_INTERP2_FAST=0 / 2), give the oracle's bits — including special queries in the
-    sorted stream."""
+    locality probe (cell-sorted queries -> the straight-line kernel, random queries -> the generic one): both choices
+    give the oracle's bits — including special queries in the sorted stream."""
     import torch
     rng = np.random.default_rng(43)
     n = 1300
@@ -464,16 +433,12 @@ def test_interp2_locality_probe_both_kernels_same_bits(b200, oracle, y_first, mo
     order = np.argsort(np.nan_to_num(cell), kind="stable")
     flags = b200.Interp2Plan.FORCE_TILES | (b200.Interp2Plan.ORDER_YX if y_first else 0)
     ref = oracle.interp2_scattered(x, y, z, xq, yq, extrap=2.5, nthreads=8, y_first=y_first)
-    for mode in ("1", "0", "2"):
-        monkeypatch.setenv("B200_INTERP2_FAST", mode)
-        if mode != "1":
-            continue   # the setting is read once per process; the forced modes are covered by tools/interp2_fast_ab.py
-        plan = b200.Interp2Plan(x, y, z, flags=flags)
-        for idx in (np.arange(nq), order):
-            tx, ty = torch.from_numpy(xq[idx]).cuda(), torch.from_numpy(yq[idx]).cuda()
-            zq = plan.scattered(tx, ty, extrap=2.5)
-            torch.cuda.synchronize()
-            assert same_bits(zq.cpu().numpy(), ref[idx])
+    plan = b200.Interp2Plan(x, y, z, flags=flags)
+    for idx in (np.arange(nq), order):
+        tx, ty = torch.from_numpy(xq[idx]).cuda(), torch.from_numpy(yq[idx]).cuda()
+        zq = plan.scattered(tx, ty, extrap=2.5)
+        torch.cuda.synchronize()
+        assert same_bits(zq.cpu().numpy(), ref[idx])
 
 
 def test_plans_run_on_their_own_device_and_restore_the_callers(b200, oracle):
