@@ -168,6 +168,20 @@ interp1_smem_kernel(AxisDev<T> ax, const T* __restrict__ yg, const T* __restrict
   }
 }
 
+// Value tables of a plan from Y at `y` (device memory): the plan's copy of Y that the shared-memory path stages
+// (yg; nullptr when Y was uploaded there directly) and one segment record (x[a], x[b], y[a], y[b]) per knot.
+template <typename T>
+__global__ void interp1_values_kernel(const T* __restrict__ x, const T* __restrict__ y, int n, T* __restrict__ yg,
+                                      T* __restrict__ seg) {
+  const int a = blockIdx.x * blockDim.x + threadIdx.x;
+  if (a >= n) return;
+  const int b = min(a + 1, n - 1);
+  const T ya = y[a];
+  if (yg) yg[a] = ya;
+  const T v[4] = {x[a], x[b], ya, y[b]};
+  st_vec4(seg + 4 * (size_t)a, v);
+}
+
 }  // namespace
 }  // namespace b200
 
@@ -199,11 +213,13 @@ template <typename T> Axis<T>& axis_of(b200_interp1_plan* p);
 template <> Axis<double>& axis_of<double>(b200_interp1_plan* p) { return p->ax64; }
 template <> Axis<float>& axis_of<float>(b200_interp1_plan* p) { return p->ax32; }
 
+// The plan's value tables from Y at `y` (device memory) on `st`; write_y: also copy Y into p->yg (the host-buffer
+// paths upload it there and pass y == p->yg).  No allocation, no host synchronisation.
 template <typename T>
-int plan1_build_seg(b200_interp1_plan* p, cudaStream_t st) {
+int plan1_build_values(b200_interp1_plan* p, const T* y, bool write_y, cudaStream_t st) {
   Axis<T>& A = axis_of<T>(p);
-  build_seg1_kernel<T><<<grid_for(p->ng), kThreads, 0, B200_CNT(st)>>>(A.x, (const T*)p->yg, (int)p->ng,
-                                                             (T*)p->seg);
+  interp1_values_kernel<T><<<grid_for(p->ng), kThreads, 0, B200_CNT(st)>>>(A.x, y, (int)p->ng,
+                                                                          write_y ? (T*)p->yg : nullptr, (T*)p->seg);
   B200_CUDA(cudaGetLastError());
   return B200_OK;
 }
@@ -219,7 +235,7 @@ int plan1_create(b200_interp1_plan* p, const T* xg, const T* yg, size_t ng) {
   B200_CUDA(cudaMemsetAsync(p->yg, 0, ng * sizeof(T) + 16, p->stream[0]));
   B200_CUDA(cudaMalloc(&p->seg, ng * 4 * sizeof(T)));
   B200_CUDA(cudaMemcpyAsync(p->yg, yg, ng * sizeof(T), cudaMemcpyHostToDevice, p->stream[0]));
-  B200_TRY(plan1_build_seg<T>(p, p->stream[0]));
+  B200_TRY(plan1_build_values<T>(p, (const T*)p->yg, false, p->stream[0]));
   B200_CUDA(cudaStreamSynchronize(p->stream[0]));
   {
     auto pad16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
@@ -378,9 +394,18 @@ int b200_interp1_plan_set_values(b200_interp1_plan* p, const void* yg) {
   DeviceScope on_plan_device(p->device);
   size_t esz = p->dtype == B200_F64 ? 8 : 4;
   B200_CUDA(cudaMemcpyAsync(p->yg, yg, p->ng * esz, cudaMemcpyHostToDevice, p->stream[0]));
-  B200_TRY(p->dtype == B200_F64 ? plan1_build_seg<double>(p, p->stream[0]) : plan1_build_seg<float>(p, p->stream[0]));
+  B200_TRY(p->dtype == B200_F64 ? plan1_build_values<double>(p, (const double*)p->yg, false, p->stream[0])
+                                : plan1_build_values<float>(p, (const float*)p->yg, false, p->stream[0]));
   B200_CUDA(cudaStreamSynchronize(p->stream[0]));
   return B200_OK;
+}
+
+int b200_interp1_plan_set_values_dev(b200_interp1_plan* p, const void* yg_dev, void* stream) {
+  if (!p || !yg_dev) return fail(B200_ERR_INVALID_ARG, "interp1_plan_set_values_dev: NULL argument");
+  DeviceScope on_plan_device(p->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  return p->dtype == B200_F64 ? plan1_build_values<double>(p, (const double*)yg_dev, true, st)
+                              : plan1_build_values<float>(p, (const float*)yg_dev, true, st);
 }
 
 int b200_interp1_plan_destroy(b200_interp1_plan* p) {

@@ -103,12 +103,17 @@ class Interp1Plan {
 
 class Interp2Plan {
  public:
-  Interp2Plan(const arma::vec& X, const arma::vec& Y, const arma::mat& Z, unsigned flags = 0) : p_(NULL) {
-    if (X.n_elem != Z.n_cols || Y.n_elem != Z.n_rows)
-      throw std::logic_error("b200::Interp2Plan: X.n_elem must equal Z.n_cols and Y.n_elem must equal Z.n_rows");
+  Interp2Plan(const arma::vec& X, const arma::vec& Y, const arma::mat& Z, unsigned flags = 0)
+      : p_(NULL), nx_(X.n_elem), ny_(Y.n_elem) {
+    CheckShape(Z);
     detail::check(b200_interp2_plan_create_ex(B200_F64, X.memptr(), X.n_elem, Y.memptr(), Y.n_elem, Z.memptr(), flags, &p_));
   }
   ~Interp2Plan() { b200_interp2_plan_destroy(p_); }
+  // new Z (Y.n_elem x X.n_elem) on the same axes; same results as a plan created with it
+  void SetValues(const arma::mat& Z) {
+    CheckShape(Z);
+    detail::check(b200_interp2_plan_set_values(p_, Z.memptr()));
+  }
   void Grid(const arma::vec& XI, const arma::vec& YI, arma::mat& ZI, double extrapolation_value = arma::datum::nan) const {
     ZI.set_size(YI.n_elem, XI.n_elem);
     detail::check(b200_interp2_grid(p_, XI.memptr(), XI.n_elem, YI.memptr(), YI.n_elem, ZI.memptr(), extrapolation_value));
@@ -124,7 +129,12 @@ class Interp2Plan {
  private:
   Interp2Plan(const Interp2Plan&);
   Interp2Plan& operator=(const Interp2Plan&);
+  void CheckShape(const arma::mat& Z) const {
+    if (nx_ != Z.n_cols || ny_ != Z.n_rows)
+      throw std::logic_error("b200::Interp2Plan: X.n_elem must equal Z.n_cols and Y.n_elem must equal Z.n_rows");
+  }
   b200_interp2_plan* p_;
+  arma::uword nx_, ny_;
 };
 
 }  // namespace b200

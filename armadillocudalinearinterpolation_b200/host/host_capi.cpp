@@ -370,4 +370,25 @@ int b200_host_interp2(const double* x, int nx, const double* y, int ny, const do
   } catch (const std::exception& e) { g_err = e.what(); return -1; }
 }
 
+// Interp2Plan from Z1 (ny x nx), then SetValues with Z2 (z2_rows x z2_cols, column-major), then Scattered at nq
+// points (xq[k], yq[k]) -> zq[k]
+int b200_host_interp2_set_values(const double* x, int nx, const double* y, int ny, const double* z1_colmajor,
+                                 const double* z2_colmajor, int z2_rows, int z2_cols, const double* xq,
+                                 const double* yq, int nq, double* zq, double extrap) {
+  try {
+    arma::vec X(nx), Y(ny), XQ(nq), YQ(nq), ZQ;
+    arma::mat Z1(ny, nx), Z2(z2_rows, z2_cols);
+    for (int i = 0; i < nx; ++i) X(i) = x[i];
+    for (int i = 0; i < ny; ++i) Y(i) = y[i];
+    for (int i = 0; i < nx * ny; ++i) Z1.memptr()[i] = z1_colmajor[i];
+    for (int i = 0; i < z2_rows * z2_cols; ++i) Z2.memptr()[i] = z2_colmajor[i];
+    for (int i = 0; i < nq; ++i) { XQ(i) = xq[i]; YQ(i) = yq[i]; }
+    b200::Interp2Plan plan(X, Y, Z1);
+    plan.SetValues(Z2);
+    plan.Scattered(XQ, YQ, ZQ, extrap);
+    for (int i = 0; i < nq; ++i) zq[i] = ZQ(i);
+    return 0;
+  } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
 }  // extern "C"

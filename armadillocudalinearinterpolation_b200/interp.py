@@ -56,6 +56,17 @@ class Interp1Plan:
         return _lib.lib().b200_interp1_plan_lookup_mode(self._h)
 
     def set_values(self, Y):
+        """New values on the same knots.  A CUDA tensor (plan dtype, contiguous, Y.numel() == n) is read in place,
+        ordered on torch's current stream; anything else is a host array (synchronous)."""
+        if _is_torch(Y) and Y.is_cuda:
+            import torch
+            tdt = torch.float64 if self.dtype == np.float64 else torch.float32
+            if Y.dtype != tdt or not Y.is_contiguous():
+                raise TypeError("device values must be a contiguous CUDA tensor of the plan's dtype")
+            if Y.numel() != self.n:
+                raise ValueError("Y has the wrong length")
+            check(_lib.lib().b200_interp1_plan_set_values_dev(self._h, C.c_void_p(Y.data_ptr()), _torch_stream()))
+            return
         Y = _np(Y, self.dtype)
         if Y.size != self.n:
             raise ValueError("Y has the wrong length")
@@ -114,6 +125,36 @@ class Interp2Plan:
         self._h = C.c_void_p()
         check(_lib.lib().b200_interp2_plan_create_ex(_DT[X.dtype], _ptr(X), C.c_size_t(X.size), _ptr(Y),
                                                     C.c_size_t(Y.size), _ptr(Zf), C.c_uint(flags), C.byref(self._h)))
+
+    def set_values(self, Z):
+        """New Z (Y.size x X.size) on the same axes; afterwards the plan gives what a plan created with Z gives.
+        A CUDA tensor of the plan's dtype is read in place, ordered on torch's current stream: strides (1, ld) are
+        passed column-major, (ld, 1) row-major, any other layout is made contiguous first.  Anything else is a host
+        array in any memory order (synchronous)."""
+        if _is_torch(Z) and Z.is_cuda:
+            import torch
+            if tuple(Z.shape) != (self.ny, self.nx):
+                raise ValueError(f"Z must have shape {(self.ny, self.nx)} (Y.size x X.size), not {tuple(Z.shape)}")
+            if Z.dtype != (torch.float64 if self.dtype == np.float64 else torch.float32):
+                raise TypeError(f"device Z must have the plan's dtype {self.dtype}, not {Z.dtype}")
+            s0, s1 = Z.stride()
+            if s1 == 1 and s0 >= self.nx:
+                ld, row_major = s0, 1
+            elif s0 == 1 and s1 >= self.ny:
+                ld, row_major = s1, 0
+            else:
+                Z = Z.contiguous()
+                ld, row_major = self.nx, 1
+            check(_lib.lib().b200_interp2_plan_set_values_dev(self._h, C.c_void_p(Z.data_ptr()), C.c_size_t(ld),
+                                                             C.c_int(row_major), _torch_stream()))
+            return
+        Z = np.asarray(Z)
+        if Z.shape != (self.ny, self.nx):
+            raise ValueError(f"Z must have shape {(self.ny, self.nx)} (Y.size x X.size), not {Z.shape}")
+        if Z.dtype.kind not in "fiu":
+            raise TypeError(f"Z of dtype {Z.dtype} is not supported (real numbers only)")
+        Zf = np.asfortranarray(Z, dtype=self.dtype)
+        check(_lib.lib().b200_interp2_plan_set_values(self._h, _ptr(Zf)))
 
     def grid(self, XI, YI, extrap=np.nan):
         """Tensor-grid queries (Armadillo's interp2 shape): returns ZI of shape (YI.size, XI.size)."""

@@ -68,8 +68,14 @@ int b200_interp2_f32(const float* x, size_t nx, const float* y, size_t ny, const
 /* dtype selects double/float for every buffer of the plan (void* below). */
 int b200_interp1_plan_create(b200_dtype dtype, const void* xg, const void* yg, size_t ng,
                              b200_interp1_plan** plan);
-/* Replace the values Y on the same knots (a new coarse profile on an unchanged grid). */
+/* Replace the values Y on the same knots (a new coarse profile on an unchanged grid).  Host buffer; runs on the
+ * plan's internal stream and returns when the plan holds the new values. */
 int b200_interp1_plan_set_values(b200_interp1_plan* plan, const void* yg);
+/* Same from device memory (ng contiguous values of the plan's dtype), ordered on `stream`: no allocation, no host
+ * synchronisation, graph-capturable.  Work of this plan queued earlier on the same stream sees the old values, later
+ * work the new.  As for every call of a plan, the caller must not have work of the same plan in flight on another
+ * stream.  Results are bit-identical to those of a plan created with the new values. */
+int b200_interp1_plan_set_values_dev(b200_interp1_plan* plan, const void* yg_dev, void* stream);
 int b200_interp1_plan_destroy(b200_interp1_plan* plan);
 
 /* Host-buffer execution: H2D of xi, kernel, D2H of yi (and idx) inside the call, chunked
@@ -111,6 +117,19 @@ int b200_interp2_plan_create(b200_dtype dtype, const void* x, size_t nx, const v
 #define B200_INTERP2_ORDER_YX 64u
 int b200_interp2_plan_create_ex(b200_dtype dtype, const void* x, size_t nx, const void* y,
                                 size_t ny, const void* z, unsigned flags, b200_interp2_plan** plan);
+/* Replace Z (ny x nx) on the same axes: a field that changes while its grid stays fixed.  The plan rebuilds its
+ * column-major Z and its scattered-query table (corner records or tiles) from the new values; the layout, the axis
+ * tables and the pass order chosen at creation stay.  Results are bit-identical to those of a plan created with the
+ * new Z (NaN and +-inf values are accepted, as at creation).
+ * Host buffer, column-major (arma::mat): synchronous, like plan creation (runs on the plan's internal stream). */
+int b200_interp2_plan_set_values(b200_interp2_plan* plan, const void* z);
+/* Same from device memory, ordered on `stream`: no allocation, no host synchronisation, graph-capturable; work of
+ * this plan queued earlier on the same stream sees the old values, later work the new.  row_major == 0: element
+ * (i, j) at j*ld + i, ld >= ny (arma::mat, or a column block of a larger one); row_major != 0: at i*ld + j, ld >= nx
+ * (a C-contiguous torch tensor of shape (ny, nx), or a row slice of a larger one).  ld below its minimum gives
+ * B200_ERR_INVALID_ARG.  The caller must not have work of the same plan in flight on another stream. */
+int b200_interp2_plan_set_values_dev(b200_interp2_plan* plan, const void* z_dev, size_t ld, int row_major,
+                                     void* stream);
 int b200_interp2_plan_destroy(b200_interp2_plan* plan);
 
 /* Tensor-grid queries (Armadillo's interp2 API shape). */
