@@ -124,6 +124,23 @@ class Interp2Plan {
     ZQ.set_size(XQ.n_elem);
     detail::check(b200_interp2_scattered(p_, XQ.memptr(), YQ.memptr(), XQ.n_elem, ZQ.memptr(), extrapolation_value));
   }
+  // Scattered plus the slopes dZ/dX, dZ/dY of the bilinear interpolant at each query (rules: b200_interp.h)
+  void ScatteredGrad(const arma::vec& XQ, const arma::vec& YQ, arma::vec& ZQ, arma::vec& DZDX, arma::vec& DZDY,
+                     double extrapolation_value = arma::datum::nan) const {
+    if (XQ.n_elem != YQ.n_elem) throw std::logic_error("b200::Interp2Plan::ScatteredGrad: XQ and YQ must have the same number of elements");
+    ZQ.set_size(XQ.n_elem);
+    DZDX.set_size(XQ.n_elem);
+    DZDY.set_size(XQ.n_elem);
+    detail::check(b200_interp2_scattered_grad(p_, XQ.memptr(), YQ.memptr(), XQ.n_elem, ZQ.memptr(), DZDX.memptr(),
+                                              DZDY.memptr(), extrapolation_value));
+  }
+  // dZ = W^T G (Y.n_elem x X.n_elem): the gradient of sum_k G(k) * ZQ(k) with respect to Z, deterministic
+  void ScatteredAdjoint(const arma::vec& XQ, const arma::vec& YQ, const arma::vec& G, arma::mat& dZ) const {
+    if (XQ.n_elem != YQ.n_elem || XQ.n_elem != G.n_elem)
+      throw std::logic_error("b200::Interp2Plan::ScatteredAdjoint: XQ, YQ and G must have the same number of elements");
+    dZ.set_size(ny_, nx_);
+    detail::check(b200_interp2_scattered_adjoint(p_, XQ.memptr(), YQ.memptr(), G.memptr(), XQ.n_elem, dZ.memptr()));
+  }
   b200_interp2_plan* handle() const { return p_; }
 
  private:

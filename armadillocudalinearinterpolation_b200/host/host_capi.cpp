@@ -391,4 +391,46 @@ int b200_host_interp2_set_values(const double* x, int nx, const double* y, int n
   } catch (const std::exception& e) { g_err = e.what(); return -1; }
 }
 
+// Interp2Plan(X, Y, Z).ScatteredGrad at nxq x-queries and nyq y-queries (different lengths are rejected):
+// zq, dzdx, dzdy get nxq entries
+int b200_host_interp2_scattered_grad(const double* x, int nx, const double* y, int ny, const double* z_colmajor,
+                                     const double* xq, int nxq, const double* yq, int nyq, double* zq, double* dzdx,
+                                     double* dzdy, double extrap) {
+  try {
+    arma::vec X(nx), Y(ny), XQ(nxq), YQ(nyq), ZQ, DX, DY;
+    arma::mat Z(ny, nx);
+    for (int i = 0; i < nx; ++i) X(i) = x[i];
+    for (int i = 0; i < ny; ++i) Y(i) = y[i];
+    for (int i = 0; i < nx * ny; ++i) Z.memptr()[i] = z_colmajor[i];
+    for (int i = 0; i < nxq; ++i) XQ(i) = xq[i];
+    for (int i = 0; i < nyq; ++i) YQ(i) = yq[i];
+    b200::Interp2Plan plan(X, Y, Z);
+    plan.ScatteredGrad(XQ, YQ, ZQ, DX, DY, extrap);
+    for (int i = 0; i < nxq; ++i) { zq[i] = ZQ(i); dzdx[i] = DX(i); dzdy[i] = DY(i); }
+    return 0;
+  } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
+// Interp2Plan(X, Y, Z).ScatteredAdjoint with nxq, nyq, ng entries of XQ, YQ, G: dz (column-major ny x nx); returns -1 with
+// the exception's text when the lengths differ or dZ comes back with another shape
+int b200_host_interp2_scattered_adjoint(const double* x, int nx, const double* y, int ny, const double* z_colmajor,
+                                        const double* xq, int nxq, const double* yq, int nyq, const double* g, int ng,
+                                        double* dz) {
+  try {
+    arma::vec X(nx), Y(ny), XQ(nxq), YQ(nyq), G(ng);
+    arma::mat Z(ny, nx), dZ;
+    for (int i = 0; i < nx; ++i) X(i) = x[i];
+    for (int i = 0; i < ny; ++i) Y(i) = y[i];
+    for (int i = 0; i < nx * ny; ++i) Z.memptr()[i] = z_colmajor[i];
+    for (int i = 0; i < nxq; ++i) XQ(i) = xq[i];
+    for (int i = 0; i < nyq; ++i) YQ(i) = yq[i];
+    for (int i = 0; i < ng; ++i) G(i) = g[i];
+    b200::Interp2Plan plan(X, Y, Z);
+    plan.ScatteredAdjoint(XQ, YQ, G, dZ);
+    if ((int)dZ.n_rows != ny || (int)dZ.n_cols != nx) { g_err = "dZ has the wrong shape"; return -1; }
+    for (int i = 0; i < nx * ny; ++i) dz[i] = dZ.memptr()[i];
+    return 0;
+  } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
 }  // extern "C"

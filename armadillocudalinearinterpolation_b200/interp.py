@@ -190,6 +190,81 @@ class Interp2Plan:
                                                C.c_double(extrap)))
         return ZQ
 
+    def _dev_queries(self, *ts):
+        """Check device operands: contiguous CUDA tensors of the plan's dtype, on one device, of equal length."""
+        import torch
+        tdt = torch.float64 if self.dtype == np.float64 else torch.float32
+        for t in ts:
+            if not (_is_torch(t) and t.is_cuda):
+                raise TypeError("device operands must all be CUDA tensors")
+            if t.dtype != tdt:
+                raise TypeError(f"device operands must have the plan's dtype {self.dtype}, not {t.dtype}")
+            if not t.is_contiguous():
+                raise TypeError("device operands must be contiguous")
+            if t.device != ts[0].device:
+                raise ValueError("device operands must be on one device")
+            if t.numel() != ts[0].numel():
+                raise ValueError("XQ, YQ (and G) must have the same number of elements")
+
+    def scattered_grad(self, XQ, YQ, extrap=np.nan):
+        """Scattered queries with their gradient: returns (ZQ, DZDX, DZDY).  ZQ has the bits of scattered(); the slopes
+        are those of the bilinear cell (NaN for a NaN coordinate, 0 outside the grid, the last cell's slope on the
+        last knot; include/b200_interp.h).  CUDA tensors run on torch's current stream; numpy arrays take the host
+        path."""
+        if _is_torch(XQ) or _is_torch(YQ):
+            import torch
+            self._dev_queries(XQ, YQ)
+            ZQ, DX, DY = torch.empty_like(XQ), torch.empty_like(XQ), torch.empty_like(XQ)
+            check(_lib.lib().b200_interp2_scattered_grad_dev(
+                self._h, C.c_void_p(XQ.data_ptr()), C.c_void_p(YQ.data_ptr()), C.c_size_t(XQ.numel()),
+                C.c_void_p(ZQ.data_ptr()), C.c_void_p(DX.data_ptr()), C.c_void_p(DY.data_ptr()), C.c_double(extrap),
+                _torch_stream()))
+            return ZQ, DX, DY
+        XQ = _np(XQ, self.dtype)
+        YQ = _np(YQ, self.dtype)
+        if XQ.shape != YQ.shape:
+            raise ValueError("XQ and YQ must have the same shape")
+        ZQ, DX, DY = (np.empty(XQ.shape, self.dtype) for _ in range(3))
+        check(_lib.lib().b200_interp2_scattered_grad(self._h, _ptr(XQ), _ptr(YQ), C.c_size_t(XQ.size), _ptr(ZQ),
+                                                    _ptr(DX), _ptr(DY), C.c_double(extrap)))
+        return ZQ, DX, DY
+
+    def scattered_adjoint(self, XQ, YQ, G):
+        """dZ = W^T G, shape (ny, nx): the gradient of sum_k G[k] * ZQ[k] with respect to Z, bit-for-bit deterministic
+        (include/b200_interp.h).  From CUDA tensors: a contiguous (row-major) CUDA tensor written on torch's current
+        stream, with the scratch taken from torch's allocator.  From numpy: a Fortran-ordered array."""
+        if _is_torch(XQ) or _is_torch(YQ) or _is_torch(G):
+            import torch
+            self._dev_queries(XQ, YQ, G)
+            lib = _lib.lib()
+            nq = XQ.numel()
+            need = C.c_size_t()
+            check(lib.b200_interp2_scattered_adjoint_workspace(self._h, C.c_size_t(nq), C.byref(need)))
+            ws = torch.empty(max(need.value, 1), dtype=torch.uint8, device=XQ.device)
+            dZ = torch.empty((self.ny, self.nx), dtype=XQ.dtype, device=XQ.device)
+            check(lib.b200_interp2_scattered_adjoint_dev(
+                self._h, C.c_void_p(XQ.data_ptr()), C.c_void_p(YQ.data_ptr()), C.c_void_p(G.data_ptr()),
+                C.c_size_t(nq), C.c_void_p(dZ.data_ptr()), C.c_size_t(self.nx), C.c_int(1),
+                C.c_void_p(ws.data_ptr()), C.c_size_t(ws.numel()), _torch_stream()))
+            return dZ
+        XQ = _np(XQ, self.dtype)
+        YQ = _np(YQ, self.dtype)
+        G = _np(G, self.dtype)
+        if not (XQ.size == YQ.size == G.size):
+            raise ValueError("XQ, YQ and G must have the same number of elements")
+        dZ = np.empty((self.ny, self.nx), self.dtype, order="F")
+        check(_lib.lib().b200_interp2_scattered_adjoint(self._h, _ptr(XQ), _ptr(YQ), _ptr(G), C.c_size_t(XQ.size),
+                                                       _ptr(dZ)))
+        return dZ
+
+    def scattered_torch(self, XQ, YQ, Z=None, extrap=np.nan):
+        """Differentiable scattered interpolation of CUDA tensors (a torch.autograd.Function): gradients flow to XQ, YQ
+        and Z.  With Z given, the plan first takes Z as its values (set_values, ordered on torch's current stream) and
+        holds them afterwards.  The backward pass uses the slopes saved by the forward pass and the adjoint; it never
+        reads the plan's values, so a set_values between forward and backward does not change the gradients.  Once
+        differentiable; no gradient for extrap."""
+        return _scattered2_function().apply(XQ, YQ, Z, self, float(extrap))
+
     def close(self):
         if self._h:
             _lib.lib().b200_interp2_plan_destroy(self._h)
@@ -200,6 +275,46 @@ class Interp2Plan:
             self.close()
         except Exception:
             pass
+
+
+_SCATTERED2 = None
+
+
+def _scattered2_function():
+    """The autograd.Function of Interp2Plan.scattered_torch (built on first use: torch is imported only when needed)."""
+    global _SCATTERED2
+    if _SCATTERED2 is None:
+        import torch
+        from torch.autograd.function import once_differentiable
+
+        class Scattered2(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, XQ, YQ, Z, plan, extrap):
+                plan._dev_queries(XQ, YQ)
+                if Z is not None:
+                    plan.set_values(Z.detach())
+                ctx.plan = plan
+                if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
+                    ZQ, DX, DY = plan.scattered_grad(XQ, YQ, extrap)
+                    ctx.save_for_backward(XQ, YQ, DX, DY)
+                else:
+                    ZQ = plan.scattered(XQ, YQ, extrap)
+                    ctx.save_for_backward(XQ, YQ)
+                return ZQ
+
+            @staticmethod
+            @once_differentiable
+            def backward(ctx, g):
+                g = g.contiguous()
+                saved = ctx.saved_tensors
+                XQ, YQ = saved[0], saved[1]
+                gx = g * saved[2] if ctx.needs_input_grad[0] else None
+                gy = g * saved[3] if ctx.needs_input_grad[1] else None
+                gZ = ctx.plan.scattered_adjoint(XQ, YQ, g) if ctx.needs_input_grad[2] else None
+                return gx, gy, gZ, None, None
+
+        _SCATTERED2 = Scattered2
+    return _SCATTERED2
 
 
 def interp1(X, Y, XI, extrap=np.nan, return_index=False):

@@ -147,6 +147,39 @@ int b200_interp2_scattered_dev(b200_interp2_plan* plan, const void* xq_dev,
                                const void* yq_dev, size_t nq, void* zq_dev,
                                double extrap_val, void* stream);
 
+/* Derivatives of scattered queries.  Every operation is rounded once; the rules do not depend on the pass order.
+ * Gradient: zq exactly as b200_interp2_scattered gives it, plus dz/dx and dz/dy of the piecewise-bilinear interpolant,
+ *   dzdx = ((1-wy)*(Z(ay,bx) - Z(ay,ax)) + wy*(Z(by,bx) - Z(by,ax))) / (X[bx] - X[ax])   (dzdy mirrored).
+ * A NaN coordinate gives NaN slopes; otherwise an out-of-range coordinate gives +0 (the output is the constant
+ * extrap_val).  On the last knot of an axis the slope along it is that of the last cell (from the left); on an
+ * interior knot it is that of the cell to the right.  NaN / inf in Z propagate as IEEE arithmetic gives.
+ * The _dev call is ordered on `stream`, allocates nothing and never synchronises the host (graph-capturable); the host
+ * call is synchronous.  Served by the plan's direct kernel (the banded pipeline serves value-only calls). */
+int b200_interp2_scattered_grad(b200_interp2_plan* plan, const void* xq, const void* yq, size_t nq,
+                                void* zq, void* dzdx, void* dzdy, double extrap_val);
+int b200_interp2_scattered_grad_dev(b200_interp2_plan* plan, const void* xq_dev, const void* yq_dev, size_t nq,
+                                    void* zq_dev, void* dzdx_dev, void* dzdy_dev, double extrap_val, void* stream);
+/* Adjoint onto the grid: G = W^T g, where row k of W holds the four bilinear weights of query k (the transpose of the
+ * scattered call; the gradient of sum_k g[k]*zq[k] with respect to Z).  Only queries with both coordinates in range
+ * contribute, each with c00 = (1-wx)(1-wy) g at (ay,ax), c10 = (1-wx) wy g at (by,ax), c01 = wx (1-wy) g at (ay,bx),
+ * c11 = wx wy g at (by,bx); a zero coefficient still makes a term (0 * inf = NaN).  Deterministic: G(i,j) = +0, then its
+ * terms added one at a time in ascending (cell key ax*ny + ay, query index k, role 00/10/01/11) order — the same bits on
+ * every call, stream and graph replay.  Because that order spans the whole batch, splitting a batch into several calls
+ * and summing changes the bits: pass all queries in one call (nq <= 2^31-1).
+ * Every G(i,j) is written: at j*ld + i (row_major == 0, ld >= ny) or i*ld + j (row_major != 0, ld >= nx), as for
+ * b200_interp2_plan_set_values_dev.  Scratch is the caller's `workspace` of at least the queried size, so the _dev call
+ * allocates nothing, never synchronises the host and can be captured into a graph.  Cost: a radix sort of the cell
+ * keys plus a few streaming passes; the terms of one node are added serially, so a batch whose queries all fall in
+ * one cell is slow (correct).  NULL pointers, a short workspace, ld below its minimum or nq > 2^31-1 give
+ * B200_ERR_INVALID_ARG before any device work; grids with nx*ny >= 2^32 give B200_ERR_UNSUPPORTED. */
+int b200_interp2_scattered_adjoint_workspace(const b200_interp2_plan* plan, size_t nq, size_t* bytes);
+int b200_interp2_scattered_adjoint_dev(b200_interp2_plan* plan, const void* xq_dev, const void* yq_dev,
+                                       const void* g_dev, size_t nq, void* G_dev, size_t ld, int row_major,
+                                       void* workspace, size_t workspace_bytes, void* stream);
+/* Host buffers, G column-major ny x nx (arma::mat): allocates, runs on the plan's internal stream, synchronous. */
+int b200_interp2_scattered_adjoint(b200_interp2_plan* plan, const void* xq, const void* yq, const void* g, size_t nq,
+                                   void* G);
+
 /* Introspection for the bench: which bracket-lookup path the plan selected
  * (0 = (quasi-)uniform knots: index arithmetic + knot fix-up on one segment record per query,
  *  1 = bucket table + bounded scan / binary search on segment records,
