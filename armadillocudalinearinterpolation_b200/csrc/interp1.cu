@@ -20,6 +20,7 @@
 //             binary search only inside pathological buckets;
 //  * the blend is (1-w)*Y[a] + w*Y[b] with w = |X[a]-q| / (|X[a]-q| + |X[b]-q|), every
 //    operation individually rounded (__dmul_rn, ...), bit-identical to the CPU oracle.
+#include <cub/device/device_radix_sort.cuh>
 #include "interp_common.cuh"
 #include "host_staging.cuh"
 
@@ -182,6 +183,258 @@ __global__ void interp1_values_kernel(const T* __restrict__ x, const T* __restri
   st_vec4(seg + 4 * (size_t)a, v);
 }
 
+// ---- derivatives (tests/interp1_grad_oracle.c restates the rules of include/b200_interp.h) ----
+// Gradient: yi exactly as the value call gives it, and dydx = (Y[b'] - Y[a']) / (X[b'] - X[a']) on the segment
+// (a', b') = (a, a+1), or (n-2, n-1) on the last knot; NaN for a NaN query, +0 for any other out-of-range one.
+// Each gradient kernel is its value kernel with one more 256-bit output stream.
+
+template <typename T>
+__device__ __forceinline__ T seg_slope(T xa, T xb, T ya, T yb) { return div_rn(sub_rn(yb, ya), sub_rn(xb, xa)); }
+
+// a query on the last knot: the slope of record n-2 (out of line: rare, and it must not cost the streaming loop
+// registers)
+template <typename T>
+__device__ __noinline__ T slope_last_record(const T* __restrict__ seg, int n) {
+  const T* r = seg + 4 * (size_t)(n - 2);
+  return seg_slope(r[0], r[1], r[2], r[3]);
+}
+
+// interp1_one plus the slope, from the record the query already loads
+template <typename T>
+__device__ __forceinline__ T interp1_grad_one(const AxisDev<T>& ax, const typename Loader1<T>::type& ld,
+                                              const T* __restrict__ seg, T q, T extrap, T& dydx) {
+  if (!(q >= ax.x0 && q <= ax.xmax)) {
+    const bool nan = q != q;
+    dydx = nan ? qnan<T>() : (T)0;
+    return nan ? qnan<T>() : extrap;
+  }
+  Seg1<T> sg;
+  if (sizeof(T) == 8 && ax.mode == 0) {
+    const int k = bin_of(ax, q);
+    sg = ld(k);
+    const double xa = (double)sg.xa, xb = (double)sg.xb, qq = (double)q;
+    const double a_err = __dsub_rn(qq, xa), b_err = __dsub_rn(xb, qq), sum = __dadd_rn(a_err, b_err);
+    if ((xa <= qq) && (qq < xb) && (a_err >= 0x1p-500) && (sum <= 0x1p500)) {
+      dydx = seg_slope(sg.xa, sg.xb, sg.ya, sg.yb);
+      return blend((T)div_rn_fast(a_err, sum), sg.ya, sg.yb);
+    }
+  }
+  const int a = find_bracket(ax, ld, q, sg);
+  dydx = a + 1 < ax.n ? seg_slope(sg.xa, sg.xb, sg.ya, sg.yb) : slope_last_record<T>(seg, ax.n);
+  return blend(weight_of(sg.xa, sg.xb, q), sg.ya, sg.yb);
+}
+
+// interp1_vec_kernel with the slope stream (32-byte aligned xi / yi / dydx)
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+interp1_grad_vec_kernel(AxisDev<T> ax, const T* __restrict__ seg, const T* __restrict__ xi, T* __restrict__ yi,
+                        T* __restrict__ dydx, size_t nvec, T extrap) {
+  constexpr int V = Vec256<T>::n;
+  const auto ld = make_loader1<T>(seg);
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
+    T q[V], y[V], d[V];
+    ld_stream_256(xi + i * V, q);
+#pragma unroll
+    for (int j = 0; j < V; ++j) y[j] = interp1_grad_one<T>(ax, ld, seg, q[j], extrap, d[j]);
+    st_stream_256(yi + i * V, y);
+    st_stream_256(dydx + i * V, d);
+  }
+}
+
+// tails and unaligned buffers
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+interp1_grad_scalar_kernel(AxisDev<T> ax, const T* __restrict__ seg, const T* __restrict__ xi, T* __restrict__ yi,
+                           T* __restrict__ dydx, size_t begin, size_t end, T extrap) {
+  const auto ld = make_loader1<T>(seg);
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = begin + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < end; i += stride) {
+    T d;
+    yi[i] = interp1_grad_one<T>(ax, ld, seg, xi[i], extrap, d);
+    dydx[i] = d;
+  }
+}
+
+// the last segment's slope on a staged (or affine) axis, out of line as slope_last_record
+template <typename T>
+__device__ __noinline__ T slope_last_knot_s(const AxisSmem<T> A, const T* sy) {
+  const int a = A.n - 2;
+  const T xa = A.affine ? affine_knot(A.affine, A.x0, A.step, A.xmax, A.n, a) : A.x[a];
+  return seg_slope(xa, A.xmax, sy[a], sy[a + 1]);
+}
+
+// interp1_smem_kernel with the slope stream.  The slope comes from sy[] and the staged or recomputed knots (affine knots
+// are bit-identical to the stored ones).  find_bracket_s<T, 2>: the derivative kernels' own instance of the
+// out-of-line knot search (interp_common.cuh), so the value kernel's register allocation does not move.
+template <typename T>
+__global__ void __launch_bounds__(kSmem1Threads)
+interp1_grad_smem_kernel(AxisDev<T> ax, const T* __restrict__ yg, const T* __restrict__ xi, T* __restrict__ yi,
+                         T* __restrict__ dydx, size_t nvec, T extrap) {
+  extern __shared__ __align__(128) unsigned char smem1g[];
+  constexpr int V = Vec256<T>::n;
+  unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem1g);
+  auto pad16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
+  const size_t yb_bytes = pad16(sizeof(T) * ax.n);
+  const size_t xb_bytes = ax.affine ? 0 : yb_bytes;
+  const size_t fb_bytes = (!ax.affine && ax.mode) ? pad16(sizeof(int32_t) * ((size_t)ax.nb + 1)) : 0;
+  T* sx = reinterpret_cast<T*>(smem1g + 16);
+  T* sy = reinterpret_cast<T*>(smem1g + 16 + xb_bytes);
+  int32_t* sf = reinterpret_cast<int32_t*>(smem1g + 16 + xb_bytes + yb_bytes);
+  if (threadIdx.x == 0) mbar_init(bar, 1);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    mbar_expect_tx(bar, (unsigned)(xb_bytes + yb_bytes + fb_bytes));
+    const unsigned chunk = 16384;
+    auto copy = [&](void* dst, const void* src, size_t bytes) {
+      for (size_t o = 0; o < bytes; o += chunk)
+        tma_bulk_g2s((unsigned char*)dst + o, (const unsigned char*)src + o, (unsigned)(bytes - o < chunk ? bytes - o : chunk), bar);
+    };
+    if (xb_bytes) copy(sx, ax.x, xb_bytes);
+    copy(sy, yg, yb_bytes);
+    if (fb_bytes) copy(sf, ax.first, fb_bytes);
+  }
+  mbar_wait(bar, 0);
+  const AxisSmem<T> A = {sx, sf, ax.x0, ax.xmax, ax.inv_w, ax.n, ax.nb, ax.mode, ax.affine, ax.step};
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
+    T q[V], y[V], d[V];
+    ld_stream_256(xi + i * V, q);
+#pragma unroll
+    for (int j = 0; j < V; ++j) {
+      const T qq = q[j];
+      if (!(qq >= A.x0 && qq <= A.xmax)) {
+        const bool nan = qq != qq;
+        y[j] = nan ? qnan<T>() : extrap;
+        d[j] = nan ? qnan<T>() : (T)0;
+      } else {
+        T xa, xb;
+        const int a = find_bracket_s<T, 2>(A, qq, xa, xb);
+        const T ya = sy[a], yb = sy[min(a + 1, A.n - 1)];
+        y[j] = blend(weight_of(xa, xb, qq), ya, yb);
+        d[j] = a + 1 < A.n ? seg_slope(xa, xb, ya, yb) : slope_last_knot_s<T>(A, sy);
+      }
+    }
+    st_stream_256(yi + i * V, y);
+    st_stream_256(dydx + i * V, d);
+  }
+}
+
+// ---- adjoint G = W^T g, deterministic (no atomics) ----
+// (1) segment key a per query, sentinel n when it does not contribute; (2) stable radix sort of (key, query index);
+// (3) adjoint_offsets_kernel: off[c] = first sorted position of segment c; (4) every term written straight into
+// node-major order; (5) the blocked sum R level by level over all nodes at once.
+//
+// Node j's list at level 0 starts at S_j = off[j-1] + off[j] (off[-1] = 0): segment j-1's role-1 terms, then segment
+// j's role-0 terms, and at node n-1 both terms of each last-knot query, interleaved by query; it ends at S_{j+1}
+// (S_n = 2 off[n], every term).  Level L+1 holds the block sums of the nodes with more than B items at level L:
+// node j's start there is floor(S_j / B) + j, which leaves room for its ceil(len_j / B) sums, so every level's layout
+// is a closed form of off[] and no scan is needed between levels.
+constexpr int kAdj1B = B200_INTERP1_ADJOINT_BLOCK;
+
+// (1): the exact search on the plan's global knots, whatever the lookup mode
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+interp1_adjoint_keys_kernel(AxisDev<T> ax, const T* __restrict__ xi, uint32_t ni, uint32_t* __restrict__ keys,
+                            uint32_t* __restrict__ idx) {
+  const AxisSmem<T> A = {ax.x, ax.first, ax.x0, ax.xmax, ax.inv_w, ax.n, ax.nb, ax.mode, ax.affine, ax.step};
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < ni; i += gridDim.x * blockDim.x) {
+    const T q = xi[i];
+    uint32_t key = (uint32_t)A.n;
+    if (q >= A.x0 && q <= A.xmax) {
+      T xa, xb;
+      key = (uint32_t)find_bracket_s<T, 2>(A, q, xa, xb);
+    }
+    keys[i] = key;
+    idx[i] = i;
+  }
+}
+
+// (4): (1-w) g[k] at node a (role 0) and w g[k] at node b (role 1), each rounded once; w is the value call's weight
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+interp1_adjoint_terms_kernel(const T* __restrict__ x, int n, const T* __restrict__ xi, const T* __restrict__ g,
+                             const uint32_t* __restrict__ keys, const uint32_t* __restrict__ idx,
+                             const uint32_t* __restrict__ off, uint32_t ni, T* __restrict__ terms) {
+  for (uint32_t s = blockIdx.x * blockDim.x + threadIdx.x; s < ni; s += gridDim.x * blockDim.x) {
+    const uint32_t a = keys[s];
+    if (a >= (uint32_t)n) break;   // sorted: the sentinels are last
+    const uint32_t k = idx[s];
+    const T gk = g[k];
+    const T w = weight_of(x[a], x[min((int)a + 1, n - 1)], xi[k]);
+    const T t0 = mul_rn(sub_rn((T)1, w), gk), t1 = mul_rn(w, gk);
+    if ((int)a + 1 < n) {
+      terms[(uint64_t)off[a] + s] = t0;        // node a: after segment a-1's role-1 terms
+      terms[(uint64_t)off[a + 1] + s] = t1;    // node a+1: first its role-1 terms
+    } else {
+      const uint64_t p = 2 * (uint64_t)off[n - 1] + 2 * (uint64_t)(s - off[n - 1]);
+      terms[p] = t0;
+      terms[p + 1] = t1;
+    }
+  }
+}
+
+// start and length of node j's items at `level` (j == n: start = the level's end), and the length one level up
+__device__ __forceinline__ void adj1_node(const uint32_t* __restrict__ off, int n, int j, int level, uint64_t& start,
+                                          uint64_t& len, uint64_t& prev_len) {
+  if (j >= n) {
+    start = 2 * (uint64_t)off[n];
+    len = 0;
+  } else {
+    const uint64_t o0 = j ? off[j - 1] : 0, o1 = off[j], o2 = off[j + 1];
+    start = o0 + o1;
+    len = (o1 - o0) + (o2 - o1) + (j == n - 1 ? o2 - o1 : 0);
+  }
+  prev_len = len;
+  for (int l = 0; l < level; ++l) {
+    start = start / kAdj1B + (uint64_t)j;
+    prev_len = len;
+    len = (len + kAdj1B - 1) / kAdj1B;
+  }
+}
+
+template <typename T>
+__device__ __forceinline__ T adj1_sum(const T* __restrict__ in, uint64_t b, uint64_t e) {
+  T acc = (T)0;
+#pragma unroll 8   // (the loads of eight items in flight before their in-order adds)
+  for (uint64_t p = b; p < e; ++p) acc = add_rn(acc, __ldg(in + p));
+  return acc;
+}
+
+// (5), one level: one thread per slot u of level+1.  The slot's node j (binary search on the closed-form starts) either
+// is live at this level (more than B items): block u - start_j of its items, summed from +0, goes to out[u]; or has
+// reached at most B items here: its first slot writes G[j], the sum of those items from +0.
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+interp1_adjoint_level_kernel(const uint32_t* __restrict__ off, int n, int level, const T* __restrict__ in,
+                             T* __restrict__ out, uint64_t nslots, T* __restrict__ G) {
+  uint64_t end, len, prev;
+  adj1_node(off, n, n, level + 1, end, len, prev);
+  if (end < nslots) nslots = end;
+  for (uint64_t u = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; u < nslots; u += (uint64_t)gridDim.x * blockDim.x) {
+    int lo = 0, hi = n - 1;   // last node whose start one level up is <= u
+    while (lo < hi) {
+      const int m = (lo + hi + 1) >> 1;
+      uint64_t s1;
+      adj1_node(off, n, m, level + 1, s1, len, prev);
+      if (s1 <= u) lo = m; else hi = m - 1;
+    }
+    const int j = lo;
+    uint64_t s0, s1;
+    adj1_node(off, n, j, level, s0, len, prev);
+    s1 = s0 / kAdj1B + (uint64_t)j;
+    const uint64_t m = u - s1;
+    if (len > (uint64_t)kAdj1B) {
+      if (m * kAdj1B < len) {
+        const uint64_t b = s0 + m * kAdj1B, e = b + kAdj1B < s0 + len ? b + kAdj1B : s0 + len;
+        out[u] = adj1_sum(in, b, e);
+      }
+    } else if (m == 0 && (level == 0 || prev > (uint64_t)kAdj1B)) {
+      G[j] = adj1_sum(in, s0, s0 + len);
+    }
+  }
+}
+
 }  // namespace
 }  // namespace b200
 
@@ -202,6 +455,7 @@ struct b200_interp1_plan {
   void* st_in[2] = {nullptr, nullptr};
   void* st_out[2] = {nullptr, nullptr};
   int32_t* st_idx[2] = {nullptr, nullptr};
+  void* st_dy[2] = {nullptr, nullptr};   // the gradient call's second output
   size_t st_cap = 0;  // queries per slot
   StagePool pool;     // pinned ring for pageable host buffers
   cudaEvent_t ev[2] = {nullptr, nullptr};
@@ -301,12 +555,12 @@ int plan1_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* i
 constexpr size_t kChunk = (size_t)1 << 22;  // queries per pipeline slot
 
 template <typename T>
-int plan1_ensure_staging(b200_interp1_plan* p, size_t ni, bool want_idx) {
+int plan1_ensure_staging(b200_interp1_plan* p, size_t ni, bool want_idx, bool want_dy = false) {
   size_t cap = ni < kChunk ? ni : kChunk;
   if (cap > p->st_cap) {
     for (int s = 0; s < 2; ++s) {
-      cudaFree(p->st_in[s]); cudaFree(p->st_out[s]); cudaFree(p->st_idx[s]);
-      p->st_in[s] = p->st_out[s] = nullptr; p->st_idx[s] = nullptr;
+      cudaFree(p->st_in[s]); cudaFree(p->st_out[s]); cudaFree(p->st_idx[s]); cudaFree(p->st_dy[s]);
+      p->st_in[s] = p->st_out[s] = p->st_dy[s] = nullptr; p->st_idx[s] = nullptr;
     }
     p->st_cap = 0;
     for (int s = 0; s < 2; ++s) {
@@ -317,6 +571,9 @@ int plan1_ensure_staging(b200_interp1_plan* p, size_t ni, bool want_idx) {
   }
   if (want_idx && !p->st_idx[0]) {
     for (int s = 0; s < 2; ++s) B200_CUDA(cudaMalloc(&p->st_idx[s], p->st_cap * sizeof(int32_t)));
+  }
+  if (want_dy && !p->st_dy[0]) {
+    for (int s = 0; s < 2; ++s) B200_CUDA(cudaMalloc(&p->st_dy[s], p->st_cap * sizeof(T)));
   }
   return B200_OK;
 }
@@ -354,13 +611,140 @@ int plan1_exec_host(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t
   return B200_OK;
 }
 
+// ---- derivatives ----
+// Value + slope on device buffers: the gradient instance of the kernel plan1_launch picks, by the same rule.
+template <typename T>
+int plan1_grad_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, T* dydx, T extrap, cudaStream_t st) {
+  if (ni == 0) return B200_OK;
+  constexpr int V = Vec256<T>::n;
+  const AxisDev<T>& ax = axis_of<T>(p).dev;
+  const T* seg = (const T*)p->seg;
+  const bool aligned = (((uintptr_t)xi | (uintptr_t)yi | (uintptr_t)dydx) % 32) == 0;
+  const size_t nvec = aligned ? ni / V : 0;
+  if (nvec && p->smem_bytes && nvec >= 4096) {
+    unsigned grid = 0;
+    B200_TRY(persistent_grid(interp1_grad_smem_kernel<T>, kSmem1Threads, p->smem_bytes, p->device,
+                             (nvec + kSmem1Threads - 1) / kSmem1Threads, grid));
+    interp1_grad_smem_kernel<T><<<grid, kSmem1Threads, p->smem_bytes, B200_CNT(st)>>>(ax, (const T*)p->yg, xi, yi, dydx,
+                                                                                     nvec, extrap);
+  } else if (nvec) {
+    const size_t blocks = (nvec + kThreads - 1) / kThreads;
+    const size_t mult = blocks > (size_t)148 * 256 ? 64 : 16;
+    const int grid = (int)(blocks < (size_t)148 * mult ? blocks : (size_t)148 * mult);
+    interp1_grad_vec_kernel<T><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, dydx, nvec, extrap);
+  }
+  const size_t done = nvec * V;
+  if (done < ni)
+    interp1_grad_scalar_kernel<T><<<capped_grid(ni - done), kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, dydx, done, ni,
+                                                                                         extrap);
+  B200_CUDA(cudaGetLastError());
+  return B200_OK;
+}
+
+// Host buffers: the pinned ring for large pageable batches, else the two-slot pipeline of plan1_exec_host with one
+// more staged output.
+template <typename T>
+int plan1_grad_host(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, T* dydx, T extrap) {
+  if (ni == 0) return B200_OK;
+  if (ni >= ((size_t)1 << 21) && (host_pageable(xi) || host_pageable(yi) || host_pageable(dydx))) {
+    std::vector<StageArray> arrays = {{xi, nullptr, sizeof(T)}, {nullptr, yi, sizeof(T)}, {nullptr, dydx, sizeof(T)}};
+    return staged_run(p->pool, p->device, arrays, ni, [&](const std::vector<void*>& d, size_t n, cudaStream_t st) {
+      return plan1_grad_launch<T>(p, (const T*)d[0], n, (T*)d[1], (T*)d[2], extrap, st);
+    });
+  }
+  B200_TRY(plan1_ensure_staging<T>(p, ni, false, true));
+  const size_t cap = p->st_cap;
+  int slot = 0;
+  for (size_t off = 0; off < ni; off += cap, slot ^= 1) {
+    const size_t n = ni - off < cap ? ni - off : cap;
+    cudaStream_t st = p->stream[slot];
+    B200_CUDA(cudaMemcpyAsync(p->st_in[slot], xi + off, n * sizeof(T), cudaMemcpyHostToDevice, st));
+    B200_TRY(plan1_grad_launch<T>(p, (const T*)p->st_in[slot], n, (T*)p->st_out[slot], (T*)p->st_dy[slot], extrap, st));
+    B200_CUDA(cudaMemcpyAsync(yi + off, p->st_out[slot], n * sizeof(T), cudaMemcpyDeviceToHost, st));
+    B200_CUDA(cudaMemcpyAsync(dydx + off, p->st_dy[slot], n * sizeof(T), cudaMemcpyDeviceToHost, st));
+  }
+  B200_CUDA(cudaStreamSynchronize(p->stream[0]));
+  B200_CUDA(cudaStreamSynchronize(p->stream[1]));
+  return B200_OK;
+}
+
+// Adjoint workspace, every part 256-byte aligned: keys and query indices twice (the radix sort's double buffer), the
+// segment offsets, the 2 ni terms, the block sums of the levels above the terms, the sort's scratch.  A node holds at
+// most 2 ni items, so `passes` levels (each dividing that bound by B) bring every node to at most B items.
+constexpr int kAdj1MaxPasses = 5;
+struct Adjoint1Ws {
+  size_t keys[2], idx[2], off, terms, level[kAdj1MaxPasses], temp, temp_bytes, total;
+  uint64_t nslots[kAdj1MaxPasses];   // slots of level L+1 (an upper bound of their end), L = 0 .. passes-1
+  int end_bit, passes;
+};
+
+inline int adjoint1_ws(const b200_interp1_plan* p, size_t ni, Adjoint1Ws& w) {
+  const uint64_t n = p->ng;   // also the sentinel key
+  int bits = 0;
+  while (bits < 32 && (n >> bits) != 0) ++bits;
+  w.end_bit = bits;
+  cub::DoubleBuffer<uint32_t> k(nullptr, nullptr), v(nullptr, nullptr);
+  w.temp_bytes = 0;
+  B200_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, w.temp_bytes, k, v, (int)(ni > 1 ? ni : 2), 0, w.end_bit));
+  const size_t esz = p->dtype == B200_F64 ? 8 : 4;
+  auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  size_t o = 0;
+  for (int s = 0; s < 2; ++s) { w.keys[s] = o; o += al(ni * 4); w.idx[s] = o; o += al(ni * 4); }
+  w.off = o; o += al((size_t)(n + 1) * 4);
+  w.terms = o; o += al(2 * ni * esz);
+  uint64_t items = 2 * (uint64_t)ni, maxlen = items;
+  w.passes = 0;
+  for (;;) {
+    items = items / kAdj1B + n;   // the end of level L+1 is at most floor(end of level L / B) + n
+    w.nslots[w.passes++] = items;
+    if (maxlen <= (uint64_t)kAdj1B) break;
+    maxlen = (maxlen + kAdj1B - 1) / kAdj1B;
+    w.level[w.passes] = o;
+    o += al(items * esz);
+  }
+  w.temp = o; o += al(w.temp_bytes);
+  w.total = o;
+  return B200_OK;
+}
+
+template <typename T>
+int plan1_adjoint_launch(b200_interp1_plan* p, const T* xi, const T* g, size_t ni, T* G, void* workspace,
+                         const Adjoint1Ws& w, cudaStream_t st) {
+  unsigned char* ws = (unsigned char*)workspace;
+  const AxisDev<T>& ax = axis_of<T>(p).dev;
+  const int n = (int)p->ng;
+  const uint32_t m = (uint32_t)ni;
+  cub::DoubleBuffer<uint32_t> keys((uint32_t*)(ws + w.keys[0]), (uint32_t*)(ws + w.keys[1]));
+  cub::DoubleBuffer<uint32_t> idx((uint32_t*)(ws + w.idx[0]), (uint32_t*)(ws + w.idx[1]));
+  uint32_t* off = (uint32_t*)(ws + w.off);
+  T* terms = (T*)(ws + w.terms);
+  if (m) interp1_adjoint_keys_kernel<T><<<capped_grid(m), kThreads, 0, B200_CNT(st)>>>(ax, xi, m, keys.Current(), idx.Current());
+  if (m > 1) {
+    size_t temp_bytes = w.temp_bytes;
+    B200_CUDA(cub::DeviceRadixSort::SortPairs(ws + w.temp, temp_bytes, keys, idx, (int)m, 0, w.end_bit, st));
+  }
+  adjoint_offsets_kernel<<<capped_grid((size_t)n + 1), kThreads, 0, B200_CNT(st)>>>(keys.Current(), m, (uint64_t)n, off);
+  if (m)
+    interp1_adjoint_terms_kernel<T><<<capped_grid(m), kThreads, 0, B200_CNT(st)>>>(ax.x, n, xi, g, keys.Current(),
+                                                                                  idx.Current(), off, m, terms);
+  const T* in = terms;
+  for (int L = 0; L < w.passes; ++L) {
+    T* out = L + 1 < w.passes ? (T*)(ws + w.level[L + 1]) : nullptr;
+    interp1_adjoint_level_kernel<T><<<capped_grid(w.nslots[L]), kThreads, 0, B200_CNT(st)>>>(off, n, L, in, out,
+                                                                                             w.nslots[L], G);
+    in = out;
+  }
+  B200_CUDA(cudaGetLastError());
+  return B200_OK;
+}
+
 void plan1_free(b200_interp1_plan* p) {
   p->ax64.release();
   p->ax32.release();
   cudaFree(p->yg);
   cudaFree(p->seg);
   for (int s = 0; s < 2; ++s) {
-    cudaFree(p->st_in[s]); cudaFree(p->st_out[s]); cudaFree(p->st_idx[s]);
+    cudaFree(p->st_in[s]); cudaFree(p->st_out[s]); cudaFree(p->st_idx[s]); cudaFree(p->st_dy[s]);
     if (p->stream[s]) cudaStreamDestroy(p->stream[s]);
     if (p->ev[s]) cudaEventDestroy(p->ev[s]);
   }
@@ -436,6 +820,79 @@ int b200_interp1_exec_dev(b200_interp1_plan* p, const void* xi_dev, size_t ni, v
   return p->dtype == B200_F64
              ? plan1_launch<double>(p, (const double*)xi_dev, ni, (double*)yi_dev, idx_dev, extrap_val, st)
              : plan1_launch<float>(p, (const float*)xi_dev, ni, (float*)yi_dev, idx_dev, (float)extrap_val, st);
+}
+
+int b200_interp1_grad(b200_interp1_plan* p, const void* xi, size_t ni, void* yi, void* dydx, double extrap_val) {
+  if (!p || (ni && (!xi || !yi || !dydx))) return fail(B200_ERR_INVALID_ARG, "interp1_grad: NULL argument");
+  DeviceScope on_plan_device(p->device);
+  return p->dtype == B200_F64
+             ? plan1_grad_host<double>(p, (const double*)xi, ni, (double*)yi, (double*)dydx, extrap_val)
+             : plan1_grad_host<float>(p, (const float*)xi, ni, (float*)yi, (float*)dydx, (float)extrap_val);
+}
+
+int b200_interp1_grad_dev(b200_interp1_plan* p, const void* xi_dev, size_t ni, void* yi_dev, void* dydx_dev,
+                          double extrap_val, void* stream) {
+  if (!p || (ni && (!xi_dev || !yi_dev || !dydx_dev))) return fail(B200_ERR_INVALID_ARG, "interp1_grad_dev: NULL argument");
+  DeviceScope on_plan_device(p->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  return p->dtype == B200_F64
+             ? plan1_grad_launch<double>(p, (const double*)xi_dev, ni, (double*)yi_dev, (double*)dydx_dev, extrap_val, st)
+             : plan1_grad_launch<float>(p, (const float*)xi_dev, ni, (float*)yi_dev, (float*)dydx_dev, (float)extrap_val, st);
+}
+
+int b200_interp1_adjoint_workspace(const b200_interp1_plan* p, size_t ni, size_t* bytes) {
+  if (!p || !bytes) return fail(B200_ERR_INVALID_ARG, "interp1_adjoint_workspace: NULL argument");
+  if (ni > (size_t)INT32_MAX) return fail(B200_ERR_INVALID_ARG, "interp1_adjoint: %zu queries exceed 2^31-1", ni);
+  DeviceScope on_plan_device(p->device);
+  Adjoint1Ws w;
+  B200_TRY(adjoint1_ws(p, ni, w));
+  *bytes = w.total;
+  return B200_OK;
+}
+
+int b200_interp1_adjoint_dev(b200_interp1_plan* p, const void* xi_dev, const void* g_dev, size_t ni, void* G_dev,
+                             void* workspace, size_t workspace_bytes, void* stream) {
+  if (!p || !G_dev || !workspace || (ni && (!xi_dev || !g_dev)))
+    return fail(B200_ERR_INVALID_ARG, "interp1_adjoint_dev: NULL argument");
+  size_t need = 0;
+  B200_TRY(b200_interp1_adjoint_workspace(p, ni, &need));
+  if (workspace_bytes < need)
+    return fail(B200_ERR_INVALID_ARG, "interp1_adjoint_dev: workspace of %zu bytes is below the %zu required",
+                workspace_bytes, need);
+  DeviceScope on_plan_device(p->device);
+  Adjoint1Ws w;
+  B200_TRY(adjoint1_ws(p, ni, w));
+  cudaStream_t st = (cudaStream_t)stream;
+  return p->dtype == B200_F64
+             ? plan1_adjoint_launch<double>(p, (const double*)xi_dev, (const double*)g_dev, ni, (double*)G_dev, workspace, w, st)
+             : plan1_adjoint_launch<float>(p, (const float*)xi_dev, (const float*)g_dev, ni, (float*)G_dev, workspace, w, st);
+}
+
+int b200_interp1_adjoint(b200_interp1_plan* p, const void* xi, const void* g, size_t ni, void* G) {
+  if (!p || !G || (ni && (!xi || !g))) return fail(B200_ERR_INVALID_ARG, "interp1_adjoint: NULL argument");
+  size_t need = 0;
+  B200_TRY(b200_interp1_adjoint_workspace(p, ni, &need));
+  DeviceScope on_plan_device(p->device);
+  const size_t esz = p->dtype == B200_F64 ? 8 : 4, gbytes = p->ng * esz;
+  cudaStream_t st = p->stream[0];
+  void *dx = nullptr, *dg = nullptr, *dG = nullptr, *ws = nullptr;
+  auto run = [&]() -> int {
+    B200_CUDA(cudaMalloc(&dx, ni * esz + 1));
+    B200_CUDA(cudaMalloc(&dg, ni * esz + 1));
+    B200_CUDA(cudaMalloc(&dG, gbytes));
+    B200_CUDA(cudaMalloc(&ws, need));
+    if (ni) {
+      B200_CUDA(cudaMemcpyAsync(dx, xi, ni * esz, cudaMemcpyHostToDevice, st));
+      B200_CUDA(cudaMemcpyAsync(dg, g, ni * esz, cudaMemcpyHostToDevice, st));
+    }
+    B200_TRY(b200_interp1_adjoint_dev(p, dx, dg, ni, dG, ws, need, st));
+    B200_CUDA(cudaMemcpyAsync(G, dG, gbytes, cudaMemcpyDeviceToHost, st));
+    B200_CUDA(cudaStreamSynchronize(st));
+    return B200_OK;
+  };
+  const int rc = run();
+  cudaFree(dx); cudaFree(dg); cudaFree(dG); cudaFree(ws);
+  return rc;
 }
 
 int b200_interp1_f64(const double* xg, const double* yg, size_t ng, const double* xi, size_t ni,

@@ -83,7 +83,7 @@ inline void interp2(const arma::fvec& X, const arma::fvec& Y, const arma::fmat& 
 // Grid resident in HBM: one upload, many query batches (host buffers; pinned ones — b200_host_alloc — overlap best).
 class Interp1Plan {
  public:
-  Interp1Plan(const arma::vec& X, const arma::vec& Y) : p_(NULL) {
+  Interp1Plan(const arma::vec& X, const arma::vec& Y) : p_(NULL), n_(X.n_elem) {
     if (X.n_elem != Y.n_elem) throw std::logic_error("b200::Interp1Plan: X and Y must have the same number of elements");
     detail::check(b200_interp1_plan_create(B200_F64, X.memptr(), Y.memptr(), X.n_elem, &p_));
   }
@@ -93,12 +93,25 @@ class Interp1Plan {
     YI.set_size(XI.n_elem);
     detail::check(b200_interp1_exec(p_, XI.memptr(), XI.n_elem, YI.memptr(), NULL, extrapolation_value));
   }
+  // operator() plus the slope DYDX of the piecewise-linear interpolant at each query (rules: b200_interp.h)
+  void Grad(const arma::vec& XI, arma::vec& YI, arma::vec& DYDX, double extrapolation_value = arma::datum::nan) const {
+    YI.set_size(XI.n_elem);
+    DYDX.set_size(XI.n_elem);
+    detail::check(b200_interp1_grad(p_, XI.memptr(), XI.n_elem, YI.memptr(), DYDX.memptr(), extrapolation_value));
+  }
+  // dY = W^T G (one value per knot): the gradient of sum_k G(k) * YI(k) with respect to Y, deterministic
+  void Adjoint(const arma::vec& XI, const arma::vec& G, arma::vec& dY) const {
+    if (XI.n_elem != G.n_elem) throw std::logic_error("b200::Interp1Plan::Adjoint: XI and G must have the same number of elements");
+    dY.set_size(n_);
+    detail::check(b200_interp1_adjoint(p_, XI.memptr(), G.memptr(), XI.n_elem, dY.memptr()));
+  }
   b200_interp1_plan* handle() const { return p_; }   // for the *_dev entry points
 
  private:
   Interp1Plan(const Interp1Plan&);
   Interp1Plan& operator=(const Interp1Plan&);
   b200_interp1_plan* p_;
+  arma::uword n_;
 };
 
 class Interp2Plan {

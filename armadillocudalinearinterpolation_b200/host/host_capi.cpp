@@ -330,6 +330,39 @@ int b200_host_interp1(const double* x, const double* y, int n, const double* xi,
   } catch (const std::exception& e) { g_err = e.what(); return -1; }
 }
 
+// Interp1Plan(X, Y).Grad with nx knots and ny values (different lengths are rejected by the plan): yi, dydx get ni entries
+int b200_host_interp1_grad(const double* x, int nx, const double* y, int ny, const double* xi, int ni, double* yi,
+                           double* dydx, double extrap) {
+  try {
+    arma::vec X(nx), Y(ny), XI(ni), YI, DY;
+    for (int i = 0; i < nx; ++i) X(i) = x[i];
+    for (int i = 0; i < ny; ++i) Y(i) = y[i];
+    for (int i = 0; i < ni; ++i) XI(i) = xi[i];
+    b200::Interp1Plan plan(X, Y);
+    plan.Grad(XI, YI, DY, extrap);
+    if ((int)YI.n_elem != ni || (int)DY.n_elem != ni) { g_err = "YI or DYDX has the wrong size"; return -1; }
+    for (int i = 0; i < ni; ++i) { yi[i] = YI(i); dydx[i] = DY(i); }
+    return 0;
+  } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
+// Interp1Plan(X, Y).Adjoint with ni entries of XI and ng of G: dy (n values); returns -1 with the exception's text when
+// the lengths differ or dY comes back with another size
+int b200_host_interp1_adjoint(const double* x, const double* y, int n, const double* xi, int ni, const double* g, int ng,
+                              double* dy) {
+  try {
+    arma::vec X(n), Y(n), XI(ni), G(ng), dY;
+    for (int i = 0; i < n; ++i) { X(i) = x[i]; Y(i) = y[i]; }
+    for (int i = 0; i < ni; ++i) XI(i) = xi[i];
+    for (int i = 0; i < ng; ++i) G(i) = g[i];
+    b200::Interp1Plan plan(X, Y);
+    plan.Adjoint(XI, G, dY);
+    if ((int)dY.n_elem != n) { g_err = "dY has the wrong size"; return -1; }
+    for (int i = 0; i < n; ++i) dy[i] = dY(i);
+    return 0;
+  } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
 // arma::fvec overload of b200::interp1
 int b200_host_interp1_f32(const float* x, const float* y, int n, const float* xi, int ni, float* yi, float extrap) {
   try {

@@ -95,6 +95,73 @@ class Interp1Plan:
                                               C.c_double(extrap), _torch_stream()))
         return (YI, idx) if return_index else YI
 
+    def _dev_operands(self, *ts):
+        """Check device operands: contiguous CUDA tensors of the plan's dtype, on one device, of equal length."""
+        import torch
+        tdt = torch.float64 if self.dtype == np.float64 else torch.float32
+        for t in ts:
+            if not (_is_torch(t) and t.is_cuda):
+                raise TypeError("device operands must all be CUDA tensors")
+            if t.dtype != tdt:
+                raise TypeError(f"device operands must have the plan's dtype {self.dtype}, not {t.dtype}")
+            if not t.is_contiguous():
+                raise TypeError("device operands must be contiguous")
+            if t.device != ts[0].device:
+                raise ValueError("device operands must be on one device")
+            if t.numel() != ts[0].numel():
+                raise ValueError("XI and G must have the same number of elements")
+
+    def grad(self, XI, extrap=np.nan):
+        """Queries with their gradient: returns (YI, DYDX).  YI has the bits of the value call; DYDX is the slope of the
+        segment (NaN for a NaN query, 0 outside the grid, the last segment's slope on the last knot;
+        include/b200_interp.h).  A CUDA tensor runs on torch's current stream; numpy arrays take the host path."""
+        if _is_torch(XI):
+            import torch
+            self._dev_operands(XI)
+            YI, DY = torch.empty_like(XI), torch.empty_like(XI)
+            check(_lib.lib().b200_interp1_grad_dev(self._h, C.c_void_p(XI.data_ptr()), C.c_size_t(XI.numel()),
+                                                  C.c_void_p(YI.data_ptr()), C.c_void_p(DY.data_ptr()),
+                                                  C.c_double(extrap), _torch_stream()))
+            return YI, DY
+        XI = _np(XI, self.dtype)
+        YI, DY = np.empty(XI.shape, self.dtype), np.empty(XI.shape, self.dtype)
+        check(_lib.lib().b200_interp1_grad(self._h, _ptr(XI), C.c_size_t(XI.size), _ptr(YI), _ptr(DY),
+                                          C.c_double(extrap)))
+        return YI, DY
+
+    def adjoint(self, XI, G):
+        """dY = W^T G (n values): the gradient of sum_k G[k] * YI[k] with respect to Y, bit-for-bit deterministic
+        (include/b200_interp.h).  From CUDA tensors: a CUDA tensor written on torch's current stream, with the scratch
+        taken from torch's allocator.  From numpy: a numpy array."""
+        if _is_torch(XI) or _is_torch(G):
+            import torch
+            self._dev_operands(XI, G)
+            lib = _lib.lib()
+            ni = XI.numel()
+            need = C.c_size_t()
+            check(lib.b200_interp1_adjoint_workspace(self._h, C.c_size_t(ni), C.byref(need)))
+            ws = torch.empty(max(need.value, 1), dtype=torch.uint8, device=XI.device)
+            dY = torch.empty(self.n, dtype=XI.dtype, device=XI.device)
+            check(lib.b200_interp1_adjoint_dev(self._h, C.c_void_p(XI.data_ptr()), C.c_void_p(G.data_ptr()),
+                                              C.c_size_t(ni), C.c_void_p(dY.data_ptr()), C.c_void_p(ws.data_ptr()),
+                                              C.c_size_t(ws.numel()), _torch_stream()))
+            return dY
+        XI = _np(XI, self.dtype)
+        G = _np(G, self.dtype)
+        if XI.size != G.size:
+            raise ValueError("XI and G must have the same number of elements")
+        dY = np.empty(self.n, self.dtype)
+        check(_lib.lib().b200_interp1_adjoint(self._h, _ptr(XI), _ptr(G), C.c_size_t(XI.size), _ptr(dY)))
+        return dY
+
+    def interp_torch(self, XI, Y=None, extrap=np.nan):
+        """Differentiable interpolation of a CUDA tensor (a torch.autograd.Function): gradients flow to XI and Y.  With Y
+        given, the plan first takes Y as its values (set_values, ordered on torch's current stream) and holds them
+        afterwards.  The backward pass uses the slopes saved by the forward pass and the adjoint; it never reads the
+        plan's values, so a set_values between forward and backward does not change the gradients.  Once
+        differentiable; no gradient for extrap."""
+        return _interp1_function().apply(XI, Y, self, float(extrap))
+
     def close(self):
         if self._h:
             _lib.lib().b200_interp1_plan_destroy(self._h)
@@ -275,6 +342,44 @@ class Interp2Plan:
             self.close()
         except Exception:
             pass
+
+
+_INTERP1 = None
+
+
+def _interp1_function():
+    """The autograd.Function of Interp1Plan.interp_torch (built on first use: torch is imported only when needed)."""
+    global _INTERP1
+    if _INTERP1 is None:
+        import torch
+        from torch.autograd.function import once_differentiable
+
+        class Interp1(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, XI, Y, plan, extrap):
+                plan._dev_operands(XI)
+                if Y is not None:
+                    plan.set_values(Y.detach())
+                ctx.plan = plan
+                if ctx.needs_input_grad[0]:
+                    YI, DY = plan.grad(XI, extrap)
+                    ctx.save_for_backward(XI, DY)
+                else:
+                    YI = plan(XI, extrap)
+                    ctx.save_for_backward(XI)
+                return YI
+
+            @staticmethod
+            @once_differentiable
+            def backward(ctx, g):
+                g = g.contiguous()
+                saved = ctx.saved_tensors
+                gx = g * saved[1] if ctx.needs_input_grad[0] else None
+                gY = ctx.plan.adjoint(saved[0], g) if ctx.needs_input_grad[1] else None
+                return gx, gY, None, None
+
+        _INTERP1 = Interp1
+    return _INTERP1
 
 
 _SCATTERED2 = None

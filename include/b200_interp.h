@@ -86,6 +86,40 @@ int b200_interp1_exec(b200_interp1_plan* plan, const void* xi, size_t ni, void* 
 int b200_interp1_exec_dev(b200_interp1_plan* plan, const void* xi_dev, size_t ni,
                           void* yi_dev, int32_t* idx_dev, double extrap_val, void* stream);
 
+/* Derivatives of interp1.  Notation: a is the value call's lower bracket, b = min(a+1, n-1), w its weight; every
+ * operation is rounded once.
+ * Gradient: yi exactly as b200_interp1_exec gives it, plus the slope of the piecewise-linear interpolant,
+ *   dydx = (Y[b'] - Y[a']) / (X[b'] - X[a'])  on the segment (a', b') = (a, a+1);
+ * on the last knot (a == n-1) the segment is (n-2, n-1), from the left; on an interior knot it is the segment to the
+ * right.  A NaN query gives a NaN slope; any other out-of-range query (+-inf included) gives +0.  NaN / inf in Y
+ * propagate as IEEE arithmetic gives (the 1-D form of the interp2 rule).
+ * The _dev call is ordered on `stream`, allocates nothing and never synchronises the host (graph-capturable); the host
+ * call is synchronous. */
+int b200_interp1_grad(b200_interp1_plan* plan, const void* xi, size_t ni, void* yi, void* dydx, double extrap_val);
+int b200_interp1_grad_dev(b200_interp1_plan* plan, const void* xi_dev, size_t ni, void* yi_dev, void* dydx_dev,
+                          double extrap_val, void* stream);
+/* Adjoint onto the values: G = W^T g, the gradient of sum_k g[k]*yi[k] with respect to Y.  Only queries inside
+ * [X[0], X[n-1]] and not NaN contribute, each with two terms: (1-w)*g[k] at node a (role 0) and w*g[k] at node b
+ * (role 1); a zero coefficient still makes a term (0 * inf = NaN).  S_j, the terms of node j in ascending
+ * (segment a, query index k, role) order, is summed by the blocked sum R with B = B200_INTERP1_ADJOINT_BLOCK:
+ *   R(empty) = +0;  a list of at most B terms: +0, then the terms added left to right;
+ *   a longer list: cut into consecutive blocks of B terms counted from its start, each block reduced by R, then R of
+ *   the list of block sums.
+ * So a node with at most B terms gets exactly the one-at-a-time bits of the interp2 adjoint, and a heavily loaded node
+ * (1e8 queries on 1e3 knots) is summed in parallel.  The bits depend only on X, the queries, g and B — not on the
+ * launch, the stream or graph replay.  Because the order spans the whole batch, splitting a batch into several calls
+ * and summing changes the bits: pass all queries in one call (ni <= 2^31-1).
+ * G_dev receives all ng values, contiguous.  Scratch is the caller's `workspace` of at least the queried size, so the
+ * _dev call allocates nothing, never synchronises the host and can be captured into a graph.  Cost: a radix sort of the
+ * segment keys plus a few streaming passes.  NULL pointers, a short workspace or ni > 2^31-1 give B200_ERR_INVALID_ARG
+ * before any device work. */
+#define B200_INTERP1_ADJOINT_BLOCK 256
+int b200_interp1_adjoint_workspace(const b200_interp1_plan* plan, size_t ni, size_t* bytes);
+int b200_interp1_adjoint_dev(b200_interp1_plan* plan, const void* xi_dev, const void* g_dev, size_t ni, void* G_dev,
+                             void* workspace, size_t workspace_bytes, void* stream);
+/* Host buffers (G: ng values): allocates, runs on the plan's internal stream, synchronous. */
+int b200_interp1_adjoint(b200_interp1_plan* plan, const void* xi, const void* g, size_t ni, void* G);
+
 int b200_interp2_plan_create(b200_dtype dtype, const void* x, size_t nx, const void* y,
                              size_t ny, const void* z, b200_interp2_plan** plan);
 /* Same, with layout flags.  By default the plan also builds one 2x2 corner record per grid cell
