@@ -14,8 +14,7 @@
 namespace b200 {
 
 // NVTX range (header-only NVTX3: a no-op unless a profiler is attached) around host-side phases: the map's
-// lift / evolve / reduce / all-gather (edm.cu) and the slots of the host-buffer pipelines (interp1.cu, interp2.cu,
-// host_staging.cuh)
+// lift / evolve / reduce / all-gather (edm.cu) and the host-buffer calls of the interpolation plans (host_staging.cuh)
 struct NvtxRange {
   explicit NvtxRange(const char* name) { nvtxRangePushA(name); }
   ~NvtxRange() { nvtxRangePop(); }
@@ -58,6 +57,23 @@ inline cudaStream_t counted_stream(cudaStream_t s) { count_launch(); return s; }
     int s__ = (call);                 \
     if (s__ != B200_OK) return s__;   \
   } while (0)
+
+// Grow-only device scratch: reserve() keeps the allocation when it holds `need` bytes and replaces it otherwise.  A
+// failed allocation leaves the buffer empty (p == nullptr, bytes == 0), never with a capacity it does not have.
+struct DeviceBuffer {
+  void* p = nullptr;
+  size_t bytes = 0;
+  int reserve(size_t need) {
+    if (need <= bytes) return B200_OK;
+    release();
+    void* q = nullptr;
+    B200_CUDA(cudaMalloc(&q, need));
+    p = q;
+    bytes = need;
+    return B200_OK;
+  }
+  void release() { cudaFree(p); p = nullptr; bytes = 0; }
+};
 
 #ifdef __CUDACC__
 // ---- streaming (touch-once) 256-bit accessors: bypass L1, first to leave L2 ----

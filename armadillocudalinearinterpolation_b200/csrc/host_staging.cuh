@@ -1,12 +1,15 @@
-// host_staging.cuh — pageable host buffers through an internal pinned ring.
+// host_staging.cuh — host_run(), the one runner of every host-buffer query call of the interpolation plans
+// (b200_interp1_exec / _grad, b200_interp2_scattered / _scattered_grad).
 //
+// Pinned (or small) buffers go through a two-slot pipeline on the plan's two streams: H2D chunk -> kernel -> D2H
+// chunk, the upload of one slot overlapping the kernel and download of the other (PCIe is full duplex).
 // A plain arma::vec (or numpy array) is pageable memory: cudaMemcpyAsync on it is staged by the driver on the
 // calling thread, does not overlap with anything, and measured 5.5x slower end to end than pinned buffers
-// (profiles/r2_e2e.md).  When a host-pointer entry point is handed pageable memory it therefore runs this
-// pipeline instead: a few worker threads, each owning a stream and two slots of pinned + device chunk buffers,
-// take the chunks round-robin — memcpy the chunk's inputs into the pinned slot, H2D, kernel, D2H into the
-// pinned slot, and copy the previous chunk's outputs back to the caller while the GPU works on this one.
-// The arithmetic is the device path's own kernels on the same values: results are bit-identical.
+// (profiles/r2_e2e.md).  Large pageable batches therefore go through staged_run() instead: a few worker threads,
+// each owning a stream and two slots of pinned + device chunk buffers, take the chunks round-robin — memcpy the
+// chunk's inputs into the pinned slot, H2D, kernel, D2H into the pinned slot, and copy the previous chunk's outputs
+// back to the caller while the GPU works on this one.
+// Both run the device path's own kernels on the same values: results are bit-identical.
 #pragma once
 #include <cstdlib>
 #include <cstring>
@@ -145,6 +148,59 @@ int staged_run(StagePool& pool, int device, const std::vector<StageArray>& array
   if (spawn_failed) return fail(B200_ERR_CUDA, "staged copy: could not start the worker threads");
   for (int t = 0; t < nworkers; ++t)
     if (status[t] != B200_OK) return fail(status[t], "%s", text[t].c_str());
+  return B200_OK;
+}
+
+// Device buffers of the two-slot pipeline, one per slot and array position.  They only grow, so a plan whose calls
+// alternate between array lists (value, value + index, gradient) keeps them: position 2 holds the int32 index of one
+// call and the slope of the next.
+struct HostSlots {
+  std::vector<DeviceBuffer> buf[2];
+  void release() {
+    for (std::vector<DeviceBuffer>& s : buf)
+      for (DeviceBuffer& b : s) b.release();
+  }
+};
+
+// n queries in host memory: `arrays` (inputs and outputs, n elements each) through staged_run when any of them is
+// pageable and n >= 2^21, else through the two-slot pipeline in chunks of 2^22 queries on `streams`; returns after
+// both streams have finished.  `launch` as for staged_run.
+template <class Launch>
+int host_run(HostSlots& slots, cudaStream_t streams[2], StagePool& pool, int device, const char* label,
+             const std::vector<StageArray>& arrays, size_t n, Launch launch) {
+  if (n == 0) return B200_OK;
+  NvtxRange nvtx_call(label);
+  bool pageable = false;
+  if (n >= ((size_t)1 << 21))
+    for (const StageArray& a : arrays) pageable = pageable || host_pageable(a.in ? a.in : a.out);
+  if (pageable) return staged_run(pool, device, arrays, n, launch);
+  constexpr size_t kChunk = (size_t)1 << 22;
+  const size_t cap = n < kChunk ? n : kChunk;
+  std::vector<void*> d[2];
+  for (int s = 0; s < 2; ++s) {
+    if (slots.buf[s].size() < arrays.size()) slots.buf[s].resize(arrays.size());
+    for (size_t a = 0; a < arrays.size(); ++a) {
+      B200_TRY(slots.buf[s][a].reserve(cap * arrays[a].elem));
+      d[s].push_back(slots.buf[s][a].p);
+    }
+  }
+  int slot = 0;
+  for (size_t off = 0; off < n; off += cap, slot ^= 1) {
+    const size_t cnt = n - off < cap ? n - off : cap;
+    cudaStream_t st = streams[slot];
+    NvtxRange nvtx_slot(slot ? "slot1 h2d+kernel+d2h" : "slot0 h2d+kernel+d2h");
+    for (size_t a = 0; a < arrays.size(); ++a)
+      if (arrays[a].in)
+        B200_CUDA(cudaMemcpyAsync(d[slot][a], (const char*)arrays[a].in + off * arrays[a].elem, cnt * arrays[a].elem,
+                                  cudaMemcpyHostToDevice, st));
+    B200_TRY(launch(d[slot], cnt, st));
+    for (size_t a = 0; a < arrays.size(); ++a)
+      if (arrays[a].out)
+        B200_CUDA(cudaMemcpyAsync((char*)arrays[a].out + off * arrays[a].elem, d[slot][a], cnt * arrays[a].elem,
+                                  cudaMemcpyDeviceToHost, st));
+  }
+  B200_CUDA(cudaStreamSynchronize(streams[0]));
+  B200_CUDA(cudaStreamSynchronize(streams[1]));
   return B200_OK;
 }
 

@@ -20,7 +20,7 @@
 //             binary search only inside pathological buckets;
 //  * the blend is (1-w)*Y[a] + w*Y[b] with w = |X[a]-q| / (|X[a]-q| + |X[b]-q|), every
 //    operation individually rounded (__dmul_rn, ...), bit-identical to the CPU oracle.
-#include <cub/device/device_radix_sort.cuh>
+// Host buffers go through host_run() (host_staging.cuh), the runner interp2.cu's scattered calls share.
 #include "interp_common.cuh"
 #include "host_staging.cuh"
 
@@ -451,14 +451,8 @@ struct b200_interp1_plan {
   void* seg = nullptr;  // [ng][4] segment records
   size_t smem_bytes = 0;  // > 0: the grid fits the shared-memory path
   cudaStream_t stream[2] = {nullptr, nullptr};
-  // staging for host-buffer execution (allocated on first use)
-  void* st_in[2] = {nullptr, nullptr};
-  void* st_out[2] = {nullptr, nullptr};
-  int32_t* st_idx[2] = {nullptr, nullptr};
-  void* st_dy[2] = {nullptr, nullptr};   // the gradient call's second output
-  size_t st_cap = 0;  // queries per slot
+  HostSlots slots;    // device buffers of the host-buffer calls (host_staging.cuh)
   StagePool pool;     // pinned ring for pageable host buffers
-  cudaEvent_t ev[2] = {nullptr, nullptr};
 };
 
 namespace {
@@ -482,8 +476,6 @@ template <typename T>
 int plan1_create(b200_interp1_plan* p, const T* xg, const T* yg, size_t ng) {
   B200_CUDA(cudaStreamCreateWithFlags(&p->stream[0], cudaStreamNonBlocking));
   B200_CUDA(cudaStreamCreateWithFlags(&p->stream[1], cudaStreamNonBlocking));
-  B200_CUDA(cudaEventCreateWithFlags(&p->ev[0], cudaEventDisableTiming));
-  B200_CUDA(cudaEventCreateWithFlags(&p->ev[1], cudaEventDisableTiming));
   B200_TRY(axis_create<T>(axis_of<T>(p), xg, ng, p->stream[0], "interp1 grid", true));
   B200_CUDA(cudaMalloc(&p->yg, ng * sizeof(T) + 16));  // +16: bulk copies move whole 16-byte units
   B200_CUDA(cudaMemsetAsync(p->yg, 0, ng * sizeof(T) + 16, p->stream[0]));
@@ -499,6 +491,15 @@ int plan1_create(b200_interp1_plan* p, const T* xg, const T* yg, size_t ng) {
     p->smem_bytes = need <= 100 * 1024 ? need : 0;   // two CTAs per SM
   }
   return B200_OK;
+}
+
+// Grid of the global-table vector kernels over nvec vectors: 16 resident CTAs per SM, 64 for very large calls,
+// grid-stride beyond that.
+// measured: 1e7 queries 37.0 us with 16 CTAs per SM vs 38.9 us with 64; 1e8 queries 0.304 ms with 64 vs 0.316 ms with 16
+inline int interp1_vec_grid(size_t nvec) {
+  const size_t blocks = (nvec + kThreads - 1) / kThreads;
+  const size_t mult = blocks > (size_t)148 * 256 ? 64 : 16;
+  return (int)(blocks < (size_t)148 * mult ? blocks : (size_t)148 * mult);
 }
 
 // Launch on device buffers.  Vector path when xi/yi(/idx) are 32-byte aligned.
@@ -522,16 +523,12 @@ int plan1_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* i
     if (idx) B200_TRY(launch(interp1_smem_kernel<T, true>));
     else B200_TRY(launch(interp1_smem_kernel<T, false>));
   } else if (nvec) {
-    // a few waves of 8 resident CTAs per SM, grid-stride beyond that
-    size_t blocks = (nvec + kThreads - 1) / kThreads;
-    // measured: 1e7 queries 37.0 us with 16 CTAs per SM vs 38.9 us with 64; 1e8 queries 0.304 ms with 64 vs 0.316 ms with 16
-    const size_t mult = blocks > (size_t)148 * 256 ? 64 : 16;
-    int grid = (int)(blocks < (size_t)148 * mult ? blocks : (size_t)148 * mult);
     // back-to-back calls on one stream (a caller that batches, the chunks of the host-buffer pipeline): with the
     // programmatic-stream-serialization attribute the next grid is scheduled while this one drains and starts the
     // moment it has completed — no launch bubble between 30-60 us kernels
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = 0; cfg.stream = B200_CNT(st);
+    cfg.gridDim = dim3((unsigned)interp1_vec_grid(nvec)); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = 0;
+    cfg.stream = B200_CNT(st);
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
@@ -540,11 +537,9 @@ int plan1_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* i
     if (idx) B200_CUDA(cudaLaunchKernelEx(&cfg, interp1_vec_kernel<T, true>, ax, seg, xi, yi, idx, nvec, extrap));
     else B200_CUDA(cudaLaunchKernelEx(&cfg, interp1_vec_kernel<T, false>, ax, seg, xi, yi, no_idx, nvec, extrap));
   }
-  size_t done = nvec * V;
+  const size_t done = nvec * V;
   if (done < ni) {
-    size_t rem = ni - done;
-    size_t blocks = (rem + kThreads - 1) / kThreads;
-    int grid = (int)(blocks < (size_t)148 * 64 ? blocks : (size_t)148 * 64);
+    const int grid = capped_grid(ni - done);
     if (idx) interp1_scalar_kernel<T, true><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, idx, done, ni, extrap);
     else interp1_scalar_kernel<T, false><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, nullptr, done, ni, extrap);
   }
@@ -552,63 +547,15 @@ int plan1_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* i
   return B200_OK;
 }
 
-constexpr size_t kChunk = (size_t)1 << 22;  // queries per pipeline slot
-
-template <typename T>
-int plan1_ensure_staging(b200_interp1_plan* p, size_t ni, bool want_idx, bool want_dy = false) {
-  size_t cap = ni < kChunk ? ni : kChunk;
-  if (cap > p->st_cap) {
-    for (int s = 0; s < 2; ++s) {
-      cudaFree(p->st_in[s]); cudaFree(p->st_out[s]); cudaFree(p->st_idx[s]); cudaFree(p->st_dy[s]);
-      p->st_in[s] = p->st_out[s] = p->st_dy[s] = nullptr; p->st_idx[s] = nullptr;
-    }
-    p->st_cap = 0;
-    for (int s = 0; s < 2; ++s) {
-      B200_CUDA(cudaMalloc(&p->st_in[s], cap * sizeof(T)));
-      B200_CUDA(cudaMalloc(&p->st_out[s], cap * sizeof(T)));
-    }
-    p->st_cap = cap;
-  }
-  if (want_idx && !p->st_idx[0]) {
-    for (int s = 0; s < 2; ++s) B200_CUDA(cudaMalloc(&p->st_idx[s], p->st_cap * sizeof(int32_t)));
-  }
-  if (want_dy && !p->st_dy[0]) {
-    for (int s = 0; s < 2; ++s) B200_CUDA(cudaMalloc(&p->st_dy[s], p->st_cap * sizeof(T)));
-  }
-  return B200_OK;
-}
-
-// Host buffers: two slots, each on its own stream: H2D(chunk) -> kernel -> D2H(chunk);
-// slot s+1's upload overlaps slot s's kernel and download (PCIe is full duplex).
+// Host buffers: host_run (host_staging.cuh) with plan1_launch
 template <typename T>
 int plan1_exec_host(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* idx, T extrap) {
-  if (ni == 0) return B200_OK;
-  NvtxRange nvtx_call("interp1:exec_host");
-  if (ni >= ((size_t)1 << 21) && (host_pageable(xi) || host_pageable(yi) || host_pageable(idx))) {
-    // ordinary (pageable) arma::vec memory: pinned ring + copier threads (host_staging.cuh), same kernels
-    std::vector<StageArray> arrays = {{xi, nullptr, sizeof(T)}, {nullptr, yi, sizeof(T)}};
-    if (idx) arrays.push_back({nullptr, idx, sizeof(int32_t)});
-    return staged_run(p->pool, p->device, arrays, ni, [&](const std::vector<void*>& d, size_t n, cudaStream_t st) {
-      return plan1_launch<T>(p, (const T*)d[0], n, (T*)d[1], idx ? (int32_t*)d[2] : nullptr, extrap, st);
-    });
-  }
-  B200_TRY(plan1_ensure_staging<T>(p, ni, idx != nullptr));
-  const size_t cap = p->st_cap;
-  int slot = 0;
-  for (size_t off = 0; off < ni; off += cap, slot ^= 1) {
-    size_t n = ni - off < cap ? ni - off : cap;
-    cudaStream_t st = p->stream[slot];
-    NvtxRange nvtx_slot(slot ? "interp1:slot1 h2d+kernel+d2h" : "interp1:slot0 h2d+kernel+d2h");
-    B200_CUDA(cudaMemcpyAsync(p->st_in[slot], xi + off, n * sizeof(T), cudaMemcpyHostToDevice, st));
-    B200_TRY(plan1_launch<T>(p, (const T*)p->st_in[slot], n, (T*)p->st_out[slot],
-                             idx ? p->st_idx[slot] : nullptr, extrap, st));
-    B200_CUDA(cudaMemcpyAsync(yi + off, p->st_out[slot], n * sizeof(T), cudaMemcpyDeviceToHost, st));
-    if (idx)
-      B200_CUDA(cudaMemcpyAsync(idx + off, p->st_idx[slot], n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  }
-  B200_CUDA(cudaStreamSynchronize(p->stream[0]));
-  B200_CUDA(cudaStreamSynchronize(p->stream[1]));
-  return B200_OK;
+  std::vector<StageArray> arrays = {{xi, nullptr, sizeof(T)}, {nullptr, yi, sizeof(T)}};
+  if (idx) arrays.push_back({nullptr, idx, sizeof(int32_t)});
+  return host_run(p->slots, p->stream, p->pool, p->device, "interp1:exec_host", arrays, ni,
+                  [&](const std::vector<void*>& d, size_t n, cudaStream_t st) {
+                    return plan1_launch<T>(p, (const T*)d[0], n, (T*)d[1], idx ? (int32_t*)d[2] : nullptr, extrap, st);
+                  });
 }
 
 // ---- derivatives ----
@@ -628,10 +575,7 @@ int plan1_grad_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, T* dy
     interp1_grad_smem_kernel<T><<<grid, kSmem1Threads, p->smem_bytes, B200_CNT(st)>>>(ax, (const T*)p->yg, xi, yi, dydx,
                                                                                      nvec, extrap);
   } else if (nvec) {
-    const size_t blocks = (nvec + kThreads - 1) / kThreads;
-    const size_t mult = blocks > (size_t)148 * 256 ? 64 : 16;
-    const int grid = (int)(blocks < (size_t)148 * mult ? blocks : (size_t)148 * mult);
-    interp1_grad_vec_kernel<T><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, dydx, nvec, extrap);
+    interp1_grad_vec_kernel<T><<<interp1_vec_grid(nvec), kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, dydx, nvec, extrap);
   }
   const size_t done = nvec * V;
   if (done < ni)
@@ -641,57 +585,31 @@ int plan1_grad_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, T* dy
   return B200_OK;
 }
 
-// Host buffers: the pinned ring for large pageable batches, else the two-slot pipeline of plan1_exec_host with one
-// more staged output.
+// Host buffers: host_run (host_staging.cuh) with plan1_grad_launch
 template <typename T>
 int plan1_grad_host(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, T* dydx, T extrap) {
-  if (ni == 0) return B200_OK;
-  if (ni >= ((size_t)1 << 21) && (host_pageable(xi) || host_pageable(yi) || host_pageable(dydx))) {
-    std::vector<StageArray> arrays = {{xi, nullptr, sizeof(T)}, {nullptr, yi, sizeof(T)}, {nullptr, dydx, sizeof(T)}};
-    return staged_run(p->pool, p->device, arrays, ni, [&](const std::vector<void*>& d, size_t n, cudaStream_t st) {
-      return plan1_grad_launch<T>(p, (const T*)d[0], n, (T*)d[1], (T*)d[2], extrap, st);
-    });
-  }
-  B200_TRY(plan1_ensure_staging<T>(p, ni, false, true));
-  const size_t cap = p->st_cap;
-  int slot = 0;
-  for (size_t off = 0; off < ni; off += cap, slot ^= 1) {
-    const size_t n = ni - off < cap ? ni - off : cap;
-    cudaStream_t st = p->stream[slot];
-    B200_CUDA(cudaMemcpyAsync(p->st_in[slot], xi + off, n * sizeof(T), cudaMemcpyHostToDevice, st));
-    B200_TRY(plan1_grad_launch<T>(p, (const T*)p->st_in[slot], n, (T*)p->st_out[slot], (T*)p->st_dy[slot], extrap, st));
-    B200_CUDA(cudaMemcpyAsync(yi + off, p->st_out[slot], n * sizeof(T), cudaMemcpyDeviceToHost, st));
-    B200_CUDA(cudaMemcpyAsync(dydx + off, p->st_dy[slot], n * sizeof(T), cudaMemcpyDeviceToHost, st));
-  }
-  B200_CUDA(cudaStreamSynchronize(p->stream[0]));
-  B200_CUDA(cudaStreamSynchronize(p->stream[1]));
-  return B200_OK;
+  return host_run(p->slots, p->stream, p->pool, p->device, "interp1:grad_host",
+                  {{xi, nullptr, sizeof(T)}, {nullptr, yi, sizeof(T)}, {nullptr, dydx, sizeof(T)}}, ni,
+                  [&](const std::vector<void*>& d, size_t n, cudaStream_t st) {
+                    return plan1_grad_launch<T>(p, (const T*)d[0], n, (T*)d[1], (T*)d[2], extrap, st);
+                  });
 }
 
-// Adjoint workspace, every part 256-byte aligned: keys and query indices twice (the radix sort's double buffer), the
-// segment offsets, the 2 ni terms, the block sums of the levels above the terms, the sort's scratch.  A node holds at
-// most 2 ni items, so `passes` levels (each dividing that bound by B) bring every node to at most B items.
+// Adjoint workspace: the shared parts (AdjointWs), the 2 ni terms and the block sums of the levels above the terms.  A
+// node holds at most 2 ni items, so `passes` levels (each dividing that bound by B) bring every node to at most B items.
 constexpr int kAdj1MaxPasses = 5;
 struct Adjoint1Ws {
-  size_t keys[2], idx[2], off, terms, level[kAdj1MaxPasses], temp, temp_bytes, total;
+  AdjointWs s;
+  size_t terms, level[kAdj1MaxPasses];
   uint64_t nslots[kAdj1MaxPasses];   // slots of level L+1 (an upper bound of their end), L = 0 .. passes-1
-  int end_bit, passes;
+  int passes;
 };
 
 inline int adjoint1_ws(const b200_interp1_plan* p, size_t ni, Adjoint1Ws& w) {
   const uint64_t n = p->ng;   // also the sentinel key
-  int bits = 0;
-  while (bits < 32 && (n >> bits) != 0) ++bits;
-  w.end_bit = bits;
-  cub::DoubleBuffer<uint32_t> k(nullptr, nullptr), v(nullptr, nullptr);
-  w.temp_bytes = 0;
-  B200_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, w.temp_bytes, k, v, (int)(ni > 1 ? ni : 2), 0, w.end_bit));
+  B200_TRY(adjoint_ws(n, ni, w.s));
   const size_t esz = p->dtype == B200_F64 ? 8 : 4;
-  auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-  size_t o = 0;
-  for (int s = 0; s < 2; ++s) { w.keys[s] = o; o += al(ni * 4); w.idx[s] = o; o += al(ni * 4); }
-  w.off = o; o += al((size_t)(n + 1) * 4);
-  w.terms = o; o += al(2 * ni * esz);
+  w.terms = w.s.add(2 * ni * esz);
   uint64_t items = 2 * (uint64_t)ni, maxlen = items;
   w.passes = 0;
   for (;;) {
@@ -699,11 +617,8 @@ inline int adjoint1_ws(const b200_interp1_plan* p, size_t ni, Adjoint1Ws& w) {
     w.nslots[w.passes++] = items;
     if (maxlen <= (uint64_t)kAdj1B) break;
     maxlen = (maxlen + kAdj1B - 1) / kAdj1B;
-    w.level[w.passes] = o;
-    o += al(items * esz);
+    w.level[w.passes] = w.s.add(items * esz);
   }
-  w.temp = o; o += al(w.temp_bytes);
-  w.total = o;
   return B200_OK;
 }
 
@@ -714,19 +629,16 @@ int plan1_adjoint_launch(b200_interp1_plan* p, const T* xi, const T* g, size_t n
   const AxisDev<T>& ax = axis_of<T>(p).dev;
   const int n = (int)p->ng;
   const uint32_t m = (uint32_t)ni;
-  cub::DoubleBuffer<uint32_t> keys((uint32_t*)(ws + w.keys[0]), (uint32_t*)(ws + w.keys[1]));
-  cub::DoubleBuffer<uint32_t> idx((uint32_t*)(ws + w.idx[0]), (uint32_t*)(ws + w.idx[1]));
-  uint32_t* off = (uint32_t*)(ws + w.off);
+  const uint32_t* off = (const uint32_t*)(ws + w.s.off);
   T* terms = (T*)(ws + w.terms);
-  if (m) interp1_adjoint_keys_kernel<T><<<capped_grid(m), kThreads, 0, B200_CNT(st)>>>(ax, xi, m, keys.Current(), idx.Current());
-  if (m > 1) {
-    size_t temp_bytes = w.temp_bytes;
-    B200_CUDA(cub::DeviceRadixSort::SortPairs(ws + w.temp, temp_bytes, keys, idx, (int)m, 0, w.end_bit, st));
-  }
-  adjoint_offsets_kernel<<<capped_grid((size_t)n + 1), kThreads, 0, B200_CNT(st)>>>(keys.Current(), m, (uint64_t)n, off);
   if (m)
-    interp1_adjoint_terms_kernel<T><<<capped_grid(m), kThreads, 0, B200_CNT(st)>>>(ax.x, n, xi, g, keys.Current(),
-                                                                                  idx.Current(), off, m, terms);
+    interp1_adjoint_keys_kernel<T><<<capped_grid(m), kThreads, 0, B200_CNT(st)>>>(ax, xi, m, (uint32_t*)(ws + w.s.keys[0]),
+                                                                                 (uint32_t*)(ws + w.s.idx[0]));
+  const uint32_t *keys = nullptr, *idx = nullptr;
+  B200_TRY(adjoint_sort(ws, w.s, m, (uint64_t)n, st, keys, idx));
+  if (m)
+    interp1_adjoint_terms_kernel<T><<<capped_grid(m), kThreads, 0, B200_CNT(st)>>>(ax.x, n, xi, g, keys, idx, off, m,
+                                                                                  terms);
   const T* in = terms;
   for (int L = 0; L < w.passes; ++L) {
     T* out = L + 1 < w.passes ? (T*)(ws + w.level[L + 1]) : nullptr;
@@ -743,11 +655,9 @@ void plan1_free(b200_interp1_plan* p) {
   p->ax32.release();
   cudaFree(p->yg);
   cudaFree(p->seg);
-  for (int s = 0; s < 2; ++s) {
-    cudaFree(p->st_in[s]); cudaFree(p->st_out[s]); cudaFree(p->st_idx[s]); cudaFree(p->st_dy[s]);
-    if (p->stream[s]) cudaStreamDestroy(p->stream[s]);
-    if (p->ev[s]) cudaEventDestroy(p->ev[s]);
-  }
+  p->slots.release();
+  for (cudaStream_t s : p->stream)
+    if (s) cudaStreamDestroy(s);
   delete p;
 }
 
@@ -846,7 +756,7 @@ int b200_interp1_adjoint_workspace(const b200_interp1_plan* p, size_t ni, size_t
   DeviceScope on_plan_device(p->device);
   Adjoint1Ws w;
   B200_TRY(adjoint1_ws(p, ni, w));
-  *bytes = w.total;
+  *bytes = w.s.total;
   return B200_OK;
 }
 
@@ -873,26 +783,12 @@ int b200_interp1_adjoint(b200_interp1_plan* p, const void* xi, const void* g, si
   size_t need = 0;
   B200_TRY(b200_interp1_adjoint_workspace(p, ni, &need));
   DeviceScope on_plan_device(p->device);
-  const size_t esz = p->dtype == B200_F64 ? 8 : 4, gbytes = p->ng * esz;
+  const size_t esz = p->dtype == B200_F64 ? 8 : 4;
   cudaStream_t st = p->stream[0];
-  void *dx = nullptr, *dg = nullptr, *dG = nullptr, *ws = nullptr;
-  auto run = [&]() -> int {
-    B200_CUDA(cudaMalloc(&dx, ni * esz + 1));
-    B200_CUDA(cudaMalloc(&dg, ni * esz + 1));
-    B200_CUDA(cudaMalloc(&dG, gbytes));
-    B200_CUDA(cudaMalloc(&ws, need));
-    if (ni) {
-      B200_CUDA(cudaMemcpyAsync(dx, xi, ni * esz, cudaMemcpyHostToDevice, st));
-      B200_CUDA(cudaMemcpyAsync(dg, g, ni * esz, cudaMemcpyHostToDevice, st));
-    }
-    B200_TRY(b200_interp1_adjoint_dev(p, dx, dg, ni, dG, ws, need, st));
-    B200_CUDA(cudaMemcpyAsync(G, dG, gbytes, cudaMemcpyDeviceToHost, st));
-    B200_CUDA(cudaStreamSynchronize(st));
-    return B200_OK;
-  };
-  const int rc = run();
-  cudaFree(dx); cudaFree(dg); cudaFree(dG); cudaFree(ws);
-  return rc;
+  return adjoint_host({xi, g}, ni * esz, G, p->ng * esz, need, st,
+                      [&](const std::vector<void*>& d, void* dG, void* ws) {
+                        return b200_interp1_adjoint_dev(p, d[0], d[1], ni, dG, ws, need, st);
+                      });
 }
 
 int b200_interp1_f64(const double* xg, const double* yg, size_t ng, const double* xi, size_t ni,

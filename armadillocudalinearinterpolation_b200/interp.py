@@ -38,6 +38,23 @@ def _torch_stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+def _dev_operands(dtype, *ts):
+    """Check device operands: contiguous CUDA tensors of the plan's dtype, on one device, of equal length."""
+    import torch
+    tdt = torch.float64 if dtype == np.float64 else torch.float32
+    for t in ts:
+        if not (_is_torch(t) and t.is_cuda):
+            raise TypeError("device operands must all be CUDA tensors")
+        if t.dtype != tdt:
+            raise TypeError(f"device operands must have the plan's dtype {dtype}, not {t.dtype}")
+        if not t.is_contiguous():
+            raise TypeError("device operands must be contiguous")
+        if t.device != ts[0].device:
+            raise ValueError("device operands must be on one device")
+        if t.numel() != ts[0].numel():
+            raise ValueError("device operands must have the same number of elements")
+
+
 class Interp1Plan:
     """Grid (X, Y) resident in HBM; interpolate many query batches (b200_interp1_plan_*)."""
 
@@ -95,29 +112,13 @@ class Interp1Plan:
                                               C.c_double(extrap), _torch_stream()))
         return (YI, idx) if return_index else YI
 
-    def _dev_operands(self, *ts):
-        """Check device operands: contiguous CUDA tensors of the plan's dtype, on one device, of equal length."""
-        import torch
-        tdt = torch.float64 if self.dtype == np.float64 else torch.float32
-        for t in ts:
-            if not (_is_torch(t) and t.is_cuda):
-                raise TypeError("device operands must all be CUDA tensors")
-            if t.dtype != tdt:
-                raise TypeError(f"device operands must have the plan's dtype {self.dtype}, not {t.dtype}")
-            if not t.is_contiguous():
-                raise TypeError("device operands must be contiguous")
-            if t.device != ts[0].device:
-                raise ValueError("device operands must be on one device")
-            if t.numel() != ts[0].numel():
-                raise ValueError("XI and G must have the same number of elements")
-
     def grad(self, XI, extrap=np.nan):
         """Queries with their gradient: returns (YI, DYDX).  YI has the bits of the value call; DYDX is the slope of the
         segment (NaN for a NaN query, 0 outside the grid, the last segment's slope on the last knot;
         include/b200_interp.h).  A CUDA tensor runs on torch's current stream; numpy arrays take the host path."""
         if _is_torch(XI):
             import torch
-            self._dev_operands(XI)
+            _dev_operands(self.dtype, XI)
             YI, DY = torch.empty_like(XI), torch.empty_like(XI)
             check(_lib.lib().b200_interp1_grad_dev(self._h, C.c_void_p(XI.data_ptr()), C.c_size_t(XI.numel()),
                                                   C.c_void_p(YI.data_ptr()), C.c_void_p(DY.data_ptr()),
@@ -135,7 +136,7 @@ class Interp1Plan:
         taken from torch's allocator.  From numpy: a numpy array."""
         if _is_torch(XI) or _is_torch(G):
             import torch
-            self._dev_operands(XI, G)
+            _dev_operands(self.dtype, XI, G)
             lib = _lib.lib()
             ni = XI.numel()
             need = C.c_size_t()
@@ -257,22 +258,6 @@ class Interp2Plan:
                                                C.c_double(extrap)))
         return ZQ
 
-    def _dev_queries(self, *ts):
-        """Check device operands: contiguous CUDA tensors of the plan's dtype, on one device, of equal length."""
-        import torch
-        tdt = torch.float64 if self.dtype == np.float64 else torch.float32
-        for t in ts:
-            if not (_is_torch(t) and t.is_cuda):
-                raise TypeError("device operands must all be CUDA tensors")
-            if t.dtype != tdt:
-                raise TypeError(f"device operands must have the plan's dtype {self.dtype}, not {t.dtype}")
-            if not t.is_contiguous():
-                raise TypeError("device operands must be contiguous")
-            if t.device != ts[0].device:
-                raise ValueError("device operands must be on one device")
-            if t.numel() != ts[0].numel():
-                raise ValueError("XQ, YQ (and G) must have the same number of elements")
-
     def scattered_grad(self, XQ, YQ, extrap=np.nan):
         """Scattered queries with their gradient: returns (ZQ, DZDX, DZDY).  ZQ has the bits of scattered(); the slopes
         are those of the bilinear cell (NaN for a NaN coordinate, 0 outside the grid, the last cell's slope on the
@@ -280,7 +265,7 @@ class Interp2Plan:
         path."""
         if _is_torch(XQ) or _is_torch(YQ):
             import torch
-            self._dev_queries(XQ, YQ)
+            _dev_operands(self.dtype, XQ, YQ)
             ZQ, DX, DY = torch.empty_like(XQ), torch.empty_like(XQ), torch.empty_like(XQ)
             check(_lib.lib().b200_interp2_scattered_grad_dev(
                 self._h, C.c_void_p(XQ.data_ptr()), C.c_void_p(YQ.data_ptr()), C.c_size_t(XQ.numel()),
@@ -302,7 +287,7 @@ class Interp2Plan:
         stream, with the scratch taken from torch's allocator.  From numpy: a Fortran-ordered array."""
         if _is_torch(XQ) or _is_torch(YQ) or _is_torch(G):
             import torch
-            self._dev_queries(XQ, YQ, G)
+            _dev_operands(self.dtype, XQ, YQ, G)
             lib = _lib.lib()
             nq = XQ.numel()
             need = C.c_size_t()
@@ -357,7 +342,7 @@ def _interp1_function():
         class Interp1(torch.autograd.Function):
             @staticmethod
             def forward(ctx, XI, Y, plan, extrap):
-                plan._dev_operands(XI)
+                _dev_operands(plan.dtype, XI)
                 if Y is not None:
                     plan.set_values(Y.detach())
                 ctx.plan = plan
@@ -395,7 +380,7 @@ def _scattered2_function():
         class Scattered2(torch.autograd.Function):
             @staticmethod
             def forward(ctx, XQ, YQ, Z, plan, extrap):
-                plan._dev_queries(XQ, YQ)
+                _dev_operands(plan.dtype, XQ, YQ)
                 if Z is not None:
                     plan.set_values(Z.detach())
                 ctx.plan = plan
