@@ -32,12 +32,33 @@ template <typename T> struct Loader1;
 template <> struct Loader1<double> { using type = LoadSeg1D; };
 template <> struct Loader1<float> { using type = LoadSeg1F; };
 
+// What a call writes besides the value of each query: nothing, the bracket index (int32, -1 out of range) or the
+// slope dydx (tests/interp1_grad_oracle.c restates the rules of include/b200_interp.h): (Y[b'] - Y[a']) / (X[b'] - X[a'])
+// on the segment (a', b') = (a, a+1), or (n-2, n-1) on the last knot; NaN for a NaN query, +0 for any other
+// out-of-range one.  Out1Of<T, OUT>: the element type of that second output stream.
+enum Out1 { kValue, kIndex, kSlope };
+template <typename T, Out1 OUT> using Out1Of = std::conditional_t<OUT == kSlope, T, int32_t>;
+
 template <typename T>
+__device__ __forceinline__ T seg_slope(T xa, T xb, T ya, T yb) { return div_rn(sub_rn(yb, ya), sub_rn(xb, xa)); }
+
+// a query on the last knot: the slope of record n-2 (out of line: rare, and it must not cost the streaming loop
+// registers)
+template <typename T>
+__device__ __noinline__ T slope_last_record(const T* __restrict__ seg, int n) {
+  const T* r = seg + 4 * (size_t)(n - 2);
+  return seg_slope(r[0], r[1], r[2], r[3]);
+}
+
+// the value of one query and, by OUT, its index or its slope (from the record the query already loads) in `out`
+template <typename T, Out1 OUT>
 __device__ __forceinline__ T interp1_one(const AxisDev<T>& ax, const typename Loader1<T>::type& ld, T q, T extrap,
-                                         int32_t& idx) {
+                                         Out1Of<T, OUT>& out) {
   if (!(q >= ax.x0 && q <= ax.xmax)) {  // out of range -> extrap_val; NaN query -> NaN
-    idx = -1;
-    return (q != q) ? qnan<T>() : extrap;
+    const bool nan = q != q;
+    if (OUT == kIndex) out = -1;
+    if (OUT == kSlope) out = nan ? qnan<T>() : (T)0;
+    return nan ? qnan<T>() : extrap;
   }
   Seg1<T> sg;
   if (sizeof(T) == 8 && ax.mode == 0) {
@@ -48,11 +69,14 @@ __device__ __forceinline__ T interp1_one(const AxisDev<T>& ax, const typename Lo
     const double xa = (double)sg.xa, xb = (double)sg.xb, qq = (double)q;
     const double a_err = __dsub_rn(qq, xa), b_err = __dsub_rn(xb, qq), sum = __dadd_rn(a_err, b_err);
     if ((xa <= qq) && (qq < xb) && (a_err >= 0x1p-500) && (sum <= 0x1p500)) {
-      idx = k;
+      if (OUT == kIndex) out = k;
+      if (OUT == kSlope) out = seg_slope(sg.xa, sg.xb, sg.ya, sg.yb);
       return blend((T)div_rn_fast(a_err, sum), sg.ya, sg.yb);
     }
   }
-  idx = find_bracket(ax, ld, q, sg);
+  const int a = find_bracket(ax, ld, q, sg);
+  if (OUT == kIndex) out = a;
+  if (OUT == kSlope) out = a + 1 < ax.n ? seg_slope(sg.xa, sg.xb, sg.ya, sg.yb) : slope_last_record<T>(ld.seg, ax.n);
   return blend(weight_of(sg.xa, sg.xb, q), sg.ya, sg.yb);
 }
 
@@ -61,50 +85,57 @@ __device__ __forceinline__ typename Loader1<T>::type make_loader1(const T* seg);
 template <> __device__ __forceinline__ LoadSeg1D make_loader1<double>(const double* seg) { return {seg}; }
 template <> __device__ __forceinline__ LoadSeg1F make_loader1<float>(const float* seg) { return {seg, l2_policy_evict_last()}; }
 
+// V results of one vector iteration: yi, and the second stream of OUT (the index: 32 bytes f32 / 16 bytes f64)
+template <typename T, Out1 OUT, int V>
+__device__ __forceinline__ void st_results(T* yi, Out1Of<T, OUT>* out, const T (&y)[V], const Out1Of<T, OUT> (&o)[V]) {
+  st_stream_256(yi, y);
+  if constexpr (OUT == kSlope) st_stream_256(out, o);
+  if constexpr (OUT == kIndex) {
+    if constexpr (V == 8) st_stream_256(out, o);
+    else st_stream_128(out, o);
+  }
+}
+
 // Vector kernel: each thread owns 32 bytes of queries per iteration (4 doubles / 8 floats),
-// i.e. V independent gather chains in flight.  Requires 32-byte aligned xi / yi.
+// i.e. V independent gather chains in flight.  Requires 32-byte aligned xi / yi and `out` aligned to its vector
+// (plan1_launch).
 // (Affine axes could gather the 16-byte value pair instead of the 32-byte record; measured within +-2 %
 // of this kernel at 1e7 and 1e8 queries — the gather RATE bounds it, not the bytes — and not kept.)
-template <typename T, bool WANT_IDX>
+template <typename T, Out1 OUT>
 __global__ void __launch_bounds__(kThreads)
 interp1_vec_kernel(AxisDev<T> ax, const T* __restrict__ seg, const T* __restrict__ xi, T* __restrict__ yi,
-                   int32_t* __restrict__ idx, size_t nvec, T extrap) {
+                   Out1Of<T, OUT>* __restrict__ out, size_t nvec, T extrap) {
   constexpr int V = Vec256<T>::n;
-  // programmatic dependent launch (plan1_launch): this grid may have been scheduled while the previous kernel of
-  // the stream was still draining; nothing is read or written before that kernel has completed and flushed
-  // (a no-op for an ordinary launch), and the next launch of the stream may be scheduled from now on
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  asm volatile("griddepcontrol.launch_dependents;");
+  if (OUT != kSlope) {
+    // programmatic dependent launch (plan1_launch): this grid may have been scheduled while the previous kernel of
+    // the stream was still draining; nothing is read or written before that kernel has completed and flushed
+    // (a no-op for an ordinary launch), and the next launch of the stream may be scheduled from now on
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    asm volatile("griddepcontrol.launch_dependents;");
+  }
   const auto ld = make_loader1<T>(seg);
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
     T q[V], y[V];
-    int32_t id[V];
+    Out1Of<T, OUT> o[V];
     ld_stream_256(xi + i * V, q);
 #pragma unroll
-    for (int j = 0; j < V; ++j) y[j] = interp1_one<T>(ax, ld, q[j], extrap, id[j]);
-    st_stream_256(yi + i * V, y);
-    if (WANT_IDX) {
-      if (V == 8) {
-        st_stream_256(idx + i * V, reinterpret_cast<const int32_t(&)[8]>(id));
-      } else {
-        st_stream_128(idx + i * V, reinterpret_cast<const int32_t(&)[4]>(id));
-      }
-    }
+    for (int j = 0; j < V; ++j) y[j] = interp1_one<T, OUT>(ax, ld, q[j], extrap, o[j]);
+    st_results<T, OUT>(yi + i * V, out + i * V, y, o);
   }
 }
 
 // Scalar kernel: tails and unaligned buffers.
-template <typename T, bool WANT_IDX>
+template <typename T, Out1 OUT>
 __global__ void __launch_bounds__(kThreads)
 interp1_scalar_kernel(AxisDev<T> ax, const T* __restrict__ seg, const T* __restrict__ xi, T* __restrict__ yi,
-                      int32_t* __restrict__ idx, size_t begin, size_t end, T extrap) {
+                      Out1Of<T, OUT>* __restrict__ out, size_t begin, size_t end, T extrap) {
   const auto ld = make_loader1<T>(seg);
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = begin + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < end; i += stride) {
-    int32_t id;
-    yi[i] = interp1_one<T>(ax, ld, xi[i], extrap, id);
-    if (WANT_IDX) idx[i] = id;
+    Out1Of<T, OUT> o;
+    yi[i] = interp1_one<T, OUT>(ax, ld, xi[i], extrap, o);
+    if (OUT != kValue) out[i] = o;
   }
 }
 
@@ -116,10 +147,21 @@ interp1_scalar_kernel(AxisDev<T> ax, const T* __restrict__ seg, const T* __restr
 // instead of staged: half the shared memory, half the bank-conflicted look-ups (0.79 vs 0.74 of peak).
 constexpr int kSmem1Threads = 512;
 
-template <typename T, bool WANT_IDX>
+// the last segment's slope on a staged (or affine) axis, out of line as slope_last_record
+template <typename T>
+__device__ __noinline__ T slope_last_knot_s(const AxisSmem<T> A, const T* sy) {
+  const int a = A.n - 2;
+  const T xa = A.affine ? affine_knot(A.affine, A.x0, A.step, A.xmax, A.n, a) : A.x[a];
+  return seg_slope(xa, A.xmax, sy[a], sy[a + 1]);
+}
+
+// The slope comes from sy[] and the staged or recomputed knots (affine knots are bit-identical to the stored ones).
+// find_bracket_s<T, 2>: the slope instance's own copy of the out-of-line knot search (interp_common.cuh), so the
+// value instances' register allocation does not depend on it.
+template <typename T, Out1 OUT>
 __global__ void __launch_bounds__(kSmem1Threads)
 interp1_smem_kernel(AxisDev<T> ax, const T* __restrict__ yg, const T* __restrict__ xi, T* __restrict__ yi,
-                    int32_t* __restrict__ idx, size_t nvec, T extrap) {
+                    Out1Of<T, OUT>* __restrict__ out, size_t nvec, T extrap) {
   extern __shared__ __align__(128) unsigned char smem1[];
   constexpr int V = Vec256<T>::n;
   unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem1);
@@ -148,24 +190,30 @@ interp1_smem_kernel(AxisDev<T> ax, const T* __restrict__ yg, const T* __restrict
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
     T q[V], y[V];
-    int32_t id[V];
+    Out1Of<T, OUT> o[V];
     ld_stream_256(xi + i * V, q);
 #pragma unroll
     for (int j = 0; j < V; ++j) {
       const T qq = q[j];
-      if (!(qq >= A.x0 && qq <= A.xmax)) { id[j] = -1; y[j] = (qq != qq) ? qnan<T>() : extrap; }
-      else {
+      if (!(qq >= A.x0 && qq <= A.xmax)) {
+        const bool nan = qq != qq;
+        if (OUT == kIndex) o[j] = -1;
+        y[j] = nan ? qnan<T>() : extrap;
+        if (OUT == kSlope) o[j] = nan ? qnan<T>() : (T)0;
+      } else {
         T xa, xb;
-        const int a = find_bracket_s(A, qq, xa, xb);
-        id[j] = a;
-        y[j] = blend(weight_of(xa, xb, qq), sy[a], sy[min(a + 1, A.n - 1)]);
+        const int a = find_bracket_s<T, OUT == kSlope ? 2 : 0>(A, qq, xa, xb);
+        if (OUT == kIndex) o[j] = a;
+        if constexpr (OUT == kSlope) {   // (values before the weight here, after it below: each instance's measured schedule)
+          const T ya = sy[a], yb = sy[min(a + 1, A.n - 1)];
+          y[j] = blend(weight_of(xa, xb, qq), ya, yb);
+          o[j] = a + 1 < A.n ? seg_slope(xa, xb, ya, yb) : slope_last_knot_s<T>(A, sy);
+        } else {
+          y[j] = blend(weight_of(xa, xb, qq), sy[a], sy[min(a + 1, A.n - 1)]);
+        }
       }
     }
-    st_stream_256(yi + i * V, y);
-    if (WANT_IDX) {
-      if (V == 8) st_stream_256(idx + i * V, reinterpret_cast<const int32_t(&)[8]>(id));
-      else st_stream_128(idx + i * V, reinterpret_cast<const int32_t(&)[4]>(id));
-    }
+    st_results<T, OUT>(yi + i * V, out + i * V, y, o);
   }
 }
 
@@ -181,143 +229,6 @@ __global__ void interp1_values_kernel(const T* __restrict__ x, const T* __restri
   if (yg) yg[a] = ya;
   const T v[4] = {x[a], x[b], ya, y[b]};
   st_vec4(seg + 4 * (size_t)a, v);
-}
-
-// ---- derivatives (tests/interp1_grad_oracle.c restates the rules of include/b200_interp.h) ----
-// Gradient: yi exactly as the value call gives it, and dydx = (Y[b'] - Y[a']) / (X[b'] - X[a']) on the segment
-// (a', b') = (a, a+1), or (n-2, n-1) on the last knot; NaN for a NaN query, +0 for any other out-of-range one.
-// Each gradient kernel is its value kernel with one more 256-bit output stream.
-
-template <typename T>
-__device__ __forceinline__ T seg_slope(T xa, T xb, T ya, T yb) { return div_rn(sub_rn(yb, ya), sub_rn(xb, xa)); }
-
-// a query on the last knot: the slope of record n-2 (out of line: rare, and it must not cost the streaming loop
-// registers)
-template <typename T>
-__device__ __noinline__ T slope_last_record(const T* __restrict__ seg, int n) {
-  const T* r = seg + 4 * (size_t)(n - 2);
-  return seg_slope(r[0], r[1], r[2], r[3]);
-}
-
-// interp1_one plus the slope, from the record the query already loads
-template <typename T>
-__device__ __forceinline__ T interp1_grad_one(const AxisDev<T>& ax, const typename Loader1<T>::type& ld,
-                                              const T* __restrict__ seg, T q, T extrap, T& dydx) {
-  if (!(q >= ax.x0 && q <= ax.xmax)) {
-    const bool nan = q != q;
-    dydx = nan ? qnan<T>() : (T)0;
-    return nan ? qnan<T>() : extrap;
-  }
-  Seg1<T> sg;
-  if (sizeof(T) == 8 && ax.mode == 0) {
-    const int k = bin_of(ax, q);
-    sg = ld(k);
-    const double xa = (double)sg.xa, xb = (double)sg.xb, qq = (double)q;
-    const double a_err = __dsub_rn(qq, xa), b_err = __dsub_rn(xb, qq), sum = __dadd_rn(a_err, b_err);
-    if ((xa <= qq) && (qq < xb) && (a_err >= 0x1p-500) && (sum <= 0x1p500)) {
-      dydx = seg_slope(sg.xa, sg.xb, sg.ya, sg.yb);
-      return blend((T)div_rn_fast(a_err, sum), sg.ya, sg.yb);
-    }
-  }
-  const int a = find_bracket(ax, ld, q, sg);
-  dydx = a + 1 < ax.n ? seg_slope(sg.xa, sg.xb, sg.ya, sg.yb) : slope_last_record<T>(seg, ax.n);
-  return blend(weight_of(sg.xa, sg.xb, q), sg.ya, sg.yb);
-}
-
-// interp1_vec_kernel with the slope stream (32-byte aligned xi / yi / dydx)
-template <typename T>
-__global__ void __launch_bounds__(kThreads)
-interp1_grad_vec_kernel(AxisDev<T> ax, const T* __restrict__ seg, const T* __restrict__ xi, T* __restrict__ yi,
-                        T* __restrict__ dydx, size_t nvec, T extrap) {
-  constexpr int V = Vec256<T>::n;
-  const auto ld = make_loader1<T>(seg);
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
-    T q[V], y[V], d[V];
-    ld_stream_256(xi + i * V, q);
-#pragma unroll
-    for (int j = 0; j < V; ++j) y[j] = interp1_grad_one<T>(ax, ld, seg, q[j], extrap, d[j]);
-    st_stream_256(yi + i * V, y);
-    st_stream_256(dydx + i * V, d);
-  }
-}
-
-// tails and unaligned buffers
-template <typename T>
-__global__ void __launch_bounds__(kThreads)
-interp1_grad_scalar_kernel(AxisDev<T> ax, const T* __restrict__ seg, const T* __restrict__ xi, T* __restrict__ yi,
-                           T* __restrict__ dydx, size_t begin, size_t end, T extrap) {
-  const auto ld = make_loader1<T>(seg);
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (size_t i = begin + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < end; i += stride) {
-    T d;
-    yi[i] = interp1_grad_one<T>(ax, ld, seg, xi[i], extrap, d);
-    dydx[i] = d;
-  }
-}
-
-// the last segment's slope on a staged (or affine) axis, out of line as slope_last_record
-template <typename T>
-__device__ __noinline__ T slope_last_knot_s(const AxisSmem<T> A, const T* sy) {
-  const int a = A.n - 2;
-  const T xa = A.affine ? affine_knot(A.affine, A.x0, A.step, A.xmax, A.n, a) : A.x[a];
-  return seg_slope(xa, A.xmax, sy[a], sy[a + 1]);
-}
-
-// interp1_smem_kernel with the slope stream.  The slope comes from sy[] and the staged or recomputed knots (affine knots
-// are bit-identical to the stored ones).  find_bracket_s<T, 2>: the derivative kernels' own instance of the
-// out-of-line knot search (interp_common.cuh), so the value kernel's register allocation does not move.
-template <typename T>
-__global__ void __launch_bounds__(kSmem1Threads)
-interp1_grad_smem_kernel(AxisDev<T> ax, const T* __restrict__ yg, const T* __restrict__ xi, T* __restrict__ yi,
-                         T* __restrict__ dydx, size_t nvec, T extrap) {
-  extern __shared__ __align__(128) unsigned char smem1g[];
-  constexpr int V = Vec256<T>::n;
-  unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem1g);
-  auto pad16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
-  const size_t yb_bytes = pad16(sizeof(T) * ax.n);
-  const size_t xb_bytes = ax.affine ? 0 : yb_bytes;
-  const size_t fb_bytes = (!ax.affine && ax.mode) ? pad16(sizeof(int32_t) * ((size_t)ax.nb + 1)) : 0;
-  T* sx = reinterpret_cast<T*>(smem1g + 16);
-  T* sy = reinterpret_cast<T*>(smem1g + 16 + xb_bytes);
-  int32_t* sf = reinterpret_cast<int32_t*>(smem1g + 16 + xb_bytes + yb_bytes);
-  if (threadIdx.x == 0) mbar_init(bar, 1);
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    mbar_expect_tx(bar, (unsigned)(xb_bytes + yb_bytes + fb_bytes));
-    const unsigned chunk = 16384;
-    auto copy = [&](void* dst, const void* src, size_t bytes) {
-      for (size_t o = 0; o < bytes; o += chunk)
-        tma_bulk_g2s((unsigned char*)dst + o, (const unsigned char*)src + o, (unsigned)(bytes - o < chunk ? bytes - o : chunk), bar);
-    };
-    if (xb_bytes) copy(sx, ax.x, xb_bytes);
-    copy(sy, yg, yb_bytes);
-    if (fb_bytes) copy(sf, ax.first, fb_bytes);
-  }
-  mbar_wait(bar, 0);
-  const AxisSmem<T> A = {sx, sf, ax.x0, ax.xmax, ax.inv_w, ax.n, ax.nb, ax.mode, ax.affine, ax.step};
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
-    T q[V], y[V], d[V];
-    ld_stream_256(xi + i * V, q);
-#pragma unroll
-    for (int j = 0; j < V; ++j) {
-      const T qq = q[j];
-      if (!(qq >= A.x0 && qq <= A.xmax)) {
-        const bool nan = qq != qq;
-        y[j] = nan ? qnan<T>() : extrap;
-        d[j] = nan ? qnan<T>() : (T)0;
-      } else {
-        T xa, xb;
-        const int a = find_bracket_s<T, 2>(A, qq, xa, xb);
-        const T ya = sy[a], yb = sy[min(a + 1, A.n - 1)];
-        y[j] = blend(weight_of(xa, xb, qq), ya, yb);
-        d[j] = a + 1 < A.n ? seg_slope(xa, xb, ya, yb) : slope_last_knot_s<T>(A, sy);
-      }
-    }
-    st_stream_256(yi + i * V, y);
-    st_stream_256(dydx + i * V, d);
-  }
 }
 
 // ---- adjoint G = W^T g, deterministic (no atomics) ----
@@ -502,96 +413,63 @@ inline int interp1_vec_grid(size_t nvec) {
   return (int)(blocks < (size_t)148 * mult ? blocks : (size_t)148 * mult);
 }
 
-// Launch on device buffers.  Vector path when xi/yi(/idx) are 32-byte aligned.
+// Launch on device buffers: yi and at most one of idx / dydx.  Vector kernels when every stream is aligned to its
+// vector (32 bytes; the f64 index stream 16): the shared-memory kernel for large calls on a plan whose grid fits it,
+// the record kernel otherwise; the scalar kernel takes the tail.
 template <typename T>
-int plan1_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* idx, T extrap,
+int plan1_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* idx, T* dydx, T extrap,
                  cudaStream_t st) {
   if (ni == 0) return B200_OK;
   constexpr int V = Vec256<T>::n;
   const AxisDev<T>& ax = axis_of<T>(p).dev;
   const T* seg = (const T*)p->seg;
-  const bool aligned = (((uintptr_t)xi | (uintptr_t)yi) % 32 == 0) &&
-                       (!idx || ((uintptr_t)idx % (V == 8 ? 32 : 16) == 0));
-  size_t nvec = aligned ? ni / V : 0;
-  if (nvec && p->smem_bytes && nvec >= 4096) {
-    auto launch = [&](auto kern) -> int {
+  auto run = [&](auto mode, auto* out) -> int {
+    constexpr Out1 OUT = decltype(mode)::value;
+    const bool aligned = (((uintptr_t)xi | (uintptr_t)yi) % 32 == 0) && ((uintptr_t)out % (sizeof(*out) * V) == 0);
+    const size_t nvec = aligned ? ni / V : 0;
+    if (nvec && p->smem_bytes && nvec >= 4096) {
       unsigned grid = 0;
-      B200_TRY(persistent_grid(kern, kSmem1Threads, p->smem_bytes, p->device, (nvec + kSmem1Threads - 1) / kSmem1Threads, grid));
-      kern<<<grid, kSmem1Threads, p->smem_bytes, B200_CNT(st)>>>(ax, (const T*)p->yg, xi, yi, idx, nvec, extrap);
-      return B200_OK;
-    };
-    if (idx) B200_TRY(launch(interp1_smem_kernel<T, true>));
-    else B200_TRY(launch(interp1_smem_kernel<T, false>));
-  } else if (nvec) {
-    // back-to-back calls on one stream (a caller that batches, the chunks of the host-buffer pipeline): with the
-    // programmatic-stream-serialization attribute the next grid is scheduled while this one drains and starts the
-    // moment it has completed — no launch bubble between 30-60 us kernels
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)interp1_vec_grid(nvec)); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = 0;
-    cfg.stream = B200_CNT(st);
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    int32_t* no_idx = nullptr;
-    if (idx) B200_CUDA(cudaLaunchKernelEx(&cfg, interp1_vec_kernel<T, true>, ax, seg, xi, yi, idx, nvec, extrap));
-    else B200_CUDA(cudaLaunchKernelEx(&cfg, interp1_vec_kernel<T, false>, ax, seg, xi, yi, no_idx, nvec, extrap));
-  }
-  const size_t done = nvec * V;
-  if (done < ni) {
-    const int grid = capped_grid(ni - done);
-    if (idx) interp1_scalar_kernel<T, true><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, idx, done, ni, extrap);
-    else interp1_scalar_kernel<T, false><<<grid, kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, nullptr, done, ni, extrap);
-  }
+      B200_TRY(persistent_grid(interp1_smem_kernel<T, OUT>, kSmem1Threads, p->smem_bytes, p->device,
+                               (nvec + kSmem1Threads - 1) / kSmem1Threads, grid));
+      interp1_smem_kernel<T, OUT><<<grid, kSmem1Threads, p->smem_bytes, B200_CNT(st)>>>(ax, (const T*)p->yg, xi, yi, out,
+                                                                                      nvec, extrap);
+    } else if (nvec) {
+      // back-to-back calls on one stream (a caller that batches, the chunks of the host-buffer pipeline): with the
+      // programmatic-stream-serialization attribute the next grid is scheduled while this one drains and starts the
+      // moment it has completed — no launch bubble between 30-60 us kernels.  Only the instances that wait for the
+      // previous grid (griddepcontrol.wait) before they touch memory may be launched so: not the slope instance.
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3((unsigned)interp1_vec_grid(nvec)); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = 0;
+      cfg.stream = B200_CNT(st);
+      cudaLaunchAttribute attr[1];
+      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+      attr[0].val.programmaticStreamSerializationAllowed = 1;
+      cfg.attrs = attr; cfg.numAttrs = OUT == kSlope ? 0 : 1;
+      B200_CUDA(cudaLaunchKernelEx(&cfg, interp1_vec_kernel<T, OUT>, ax, seg, xi, yi, out, nvec, extrap));
+    }
+    const size_t done = nvec * V;
+    if (done < ni)
+      interp1_scalar_kernel<T, OUT><<<capped_grid(ni - done), kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, out, done, ni,
+                                                                                           extrap);
+    return B200_OK;
+  };
+  if (dydx) B200_TRY(run(std::integral_constant<Out1, kSlope>(), dydx));
+  else if (idx) B200_TRY(run(std::integral_constant<Out1, kIndex>(), idx));
+  else B200_TRY(run(std::integral_constant<Out1, kValue>(), idx));
   B200_CUDA(cudaGetLastError());
   return B200_OK;
 }
 
 // Host buffers: host_run (host_staging.cuh) with plan1_launch
 template <typename T>
-int plan1_exec_host(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* idx, T extrap) {
+int plan1_host(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, int32_t* idx, T* dydx, T extrap) {
   std::vector<StageArray> arrays = {{xi, nullptr, sizeof(T)}, {nullptr, yi, sizeof(T)}};
   if (idx) arrays.push_back({nullptr, idx, sizeof(int32_t)});
-  return host_run(p->slots, p->stream, p->pool, p->device, "interp1:exec_host", arrays, ni,
+  if (dydx) arrays.push_back({nullptr, dydx, sizeof(T)});
+  return host_run(p->slots, p->stream, p->pool, p->device, dydx ? "interp1:grad_host" : "interp1:exec_host", arrays, ni,
                   [&](const std::vector<void*>& d, size_t n, cudaStream_t st) {
-                    return plan1_launch<T>(p, (const T*)d[0], n, (T*)d[1], idx ? (int32_t*)d[2] : nullptr, extrap, st);
-                  });
-}
-
-// ---- derivatives ----
-// Value + slope on device buffers: the gradient instance of the kernel plan1_launch picks, by the same rule.
-template <typename T>
-int plan1_grad_launch(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, T* dydx, T extrap, cudaStream_t st) {
-  if (ni == 0) return B200_OK;
-  constexpr int V = Vec256<T>::n;
-  const AxisDev<T>& ax = axis_of<T>(p).dev;
-  const T* seg = (const T*)p->seg;
-  const bool aligned = (((uintptr_t)xi | (uintptr_t)yi | (uintptr_t)dydx) % 32) == 0;
-  const size_t nvec = aligned ? ni / V : 0;
-  if (nvec && p->smem_bytes && nvec >= 4096) {
-    unsigned grid = 0;
-    B200_TRY(persistent_grid(interp1_grad_smem_kernel<T>, kSmem1Threads, p->smem_bytes, p->device,
-                             (nvec + kSmem1Threads - 1) / kSmem1Threads, grid));
-    interp1_grad_smem_kernel<T><<<grid, kSmem1Threads, p->smem_bytes, B200_CNT(st)>>>(ax, (const T*)p->yg, xi, yi, dydx,
-                                                                                     nvec, extrap);
-  } else if (nvec) {
-    interp1_grad_vec_kernel<T><<<interp1_vec_grid(nvec), kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, dydx, nvec, extrap);
-  }
-  const size_t done = nvec * V;
-  if (done < ni)
-    interp1_grad_scalar_kernel<T><<<capped_grid(ni - done), kThreads, 0, B200_CNT(st)>>>(ax, seg, xi, yi, dydx, done, ni,
-                                                                                         extrap);
-  B200_CUDA(cudaGetLastError());
-  return B200_OK;
-}
-
-// Host buffers: host_run (host_staging.cuh) with plan1_grad_launch
-template <typename T>
-int plan1_grad_host(b200_interp1_plan* p, const T* xi, size_t ni, T* yi, T* dydx, T extrap) {
-  return host_run(p->slots, p->stream, p->pool, p->device, "interp1:grad_host",
-                  {{xi, nullptr, sizeof(T)}, {nullptr, yi, sizeof(T)}, {nullptr, dydx, sizeof(T)}}, ni,
-                  [&](const std::vector<void*>& d, size_t n, cudaStream_t st) {
-                    return plan1_grad_launch<T>(p, (const T*)d[0], n, (T*)d[1], (T*)d[2], extrap, st);
+                    return plan1_launch<T>(p, (const T*)d[0], n, (T*)d[1], idx ? (int32_t*)d[2] : nullptr,
+                                           dydx ? (T*)d[2] : nullptr, extrap, st);
                   });
 }
 
@@ -718,8 +596,8 @@ int b200_interp1_exec(b200_interp1_plan* p, const void* xi, size_t ni, void* yi,
   if (!p || (ni && (!xi || !yi))) return fail(B200_ERR_INVALID_ARG, "interp1_exec: NULL argument");
   DeviceScope on_plan_device(p->device);
   return p->dtype == B200_F64
-             ? plan1_exec_host<double>(p, (const double*)xi, ni, (double*)yi, idx_out, extrap_val)
-             : plan1_exec_host<float>(p, (const float*)xi, ni, (float*)yi, idx_out, (float)extrap_val);
+             ? plan1_host<double>(p, (const double*)xi, ni, (double*)yi, idx_out, nullptr, extrap_val)
+             : plan1_host<float>(p, (const float*)xi, ni, (float*)yi, idx_out, nullptr, (float)extrap_val);
 }
 
 int b200_interp1_exec_dev(b200_interp1_plan* p, const void* xi_dev, size_t ni, void* yi_dev,
@@ -728,16 +606,16 @@ int b200_interp1_exec_dev(b200_interp1_plan* p, const void* xi_dev, size_t ni, v
   DeviceScope on_plan_device(p->device);
   cudaStream_t st = (cudaStream_t)stream;
   return p->dtype == B200_F64
-             ? plan1_launch<double>(p, (const double*)xi_dev, ni, (double*)yi_dev, idx_dev, extrap_val, st)
-             : plan1_launch<float>(p, (const float*)xi_dev, ni, (float*)yi_dev, idx_dev, (float)extrap_val, st);
+             ? plan1_launch<double>(p, (const double*)xi_dev, ni, (double*)yi_dev, idx_dev, nullptr, extrap_val, st)
+             : plan1_launch<float>(p, (const float*)xi_dev, ni, (float*)yi_dev, idx_dev, nullptr, (float)extrap_val, st);
 }
 
 int b200_interp1_grad(b200_interp1_plan* p, const void* xi, size_t ni, void* yi, void* dydx, double extrap_val) {
   if (!p || (ni && (!xi || !yi || !dydx))) return fail(B200_ERR_INVALID_ARG, "interp1_grad: NULL argument");
   DeviceScope on_plan_device(p->device);
   return p->dtype == B200_F64
-             ? plan1_grad_host<double>(p, (const double*)xi, ni, (double*)yi, (double*)dydx, extrap_val)
-             : plan1_grad_host<float>(p, (const float*)xi, ni, (float*)yi, (float*)dydx, (float)extrap_val);
+             ? plan1_host<double>(p, (const double*)xi, ni, (double*)yi, nullptr, (double*)dydx, extrap_val)
+             : plan1_host<float>(p, (const float*)xi, ni, (float*)yi, nullptr, (float*)dydx, (float)extrap_val);
 }
 
 int b200_interp1_grad_dev(b200_interp1_plan* p, const void* xi_dev, size_t ni, void* yi_dev, void* dydx_dev,
@@ -746,8 +624,8 @@ int b200_interp1_grad_dev(b200_interp1_plan* p, const void* xi_dev, size_t ni, v
   DeviceScope on_plan_device(p->device);
   cudaStream_t st = (cudaStream_t)stream;
   return p->dtype == B200_F64
-             ? plan1_grad_launch<double>(p, (const double*)xi_dev, ni, (double*)yi_dev, (double*)dydx_dev, extrap_val, st)
-             : plan1_grad_launch<float>(p, (const float*)xi_dev, ni, (float*)yi_dev, (float*)dydx_dev, (float)extrap_val, st);
+             ? plan1_launch<double>(p, (const double*)xi_dev, ni, (double*)yi_dev, nullptr, (double*)dydx_dev, extrap_val, st)
+             : plan1_launch<float>(p, (const float*)xi_dev, ni, (float*)yi_dev, nullptr, (float*)dydx_dev, (float)extrap_val, st);
 }
 
 int b200_interp1_adjoint_workspace(const b200_interp1_plan* p, size_t ni, size_t* bytes) {
