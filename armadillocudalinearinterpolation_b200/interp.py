@@ -101,9 +101,7 @@ class Interp1Plan:
 
     def _call_dev(self, XI, extrap, return_index, out):
         import torch
-        tdt = torch.float64 if self.dtype == np.float64 else torch.float32
-        if not XI.is_cuda or XI.dtype != tdt or not XI.is_contiguous():
-            raise TypeError("device queries must be contiguous CUDA tensors of the plan's dtype")
+        _dev_operands(self.dtype, XI, *(() if out is None else (out,)))
         YI = torch.empty_like(XI) if out is None else out
         idx = torch.empty(XI.shape, dtype=torch.int32, device=XI.device) if return_index else None
         check(_lib.lib().b200_interp1_exec_dev(self._h, C.c_void_p(XI.data_ptr()), C.c_size_t(XI.numel()),
@@ -225,9 +223,14 @@ class Interp2Plan:
         check(_lib.lib().b200_interp2_plan_set_values(self._h, _ptr(Zf)))
 
     def grid(self, XI, YI, extrap=np.nan):
-        """Tensor-grid queries (Armadillo's interp2 shape): returns ZI of shape (YI.size, XI.size)."""
-        if _is_torch(XI):
+        """Tensor-grid queries (Armadillo's interp2 shape): returns ZI of shape (YI.size, XI.size).  CUDA tensors run
+        on torch's current stream; numpy arrays take the host path."""
+        if _is_torch(XI) or _is_torch(YI):
             import torch
+            _dev_operands(self.dtype, XI)
+            _dev_operands(self.dtype, YI)   # checked on its own: XI and YI may differ in length
+            if YI.device != XI.device:
+                raise ValueError("device operands must be on one device")
             ZI = torch.empty((XI.numel(), YI.numel()), dtype=XI.dtype, device=XI.device)  # column-major ZI
             check(_lib.lib().b200_interp2_grid_dev(self._h, C.c_void_p(XI.data_ptr()), C.c_size_t(XI.numel()),
                                                   C.c_void_p(YI.data_ptr()), C.c_size_t(YI.numel()),
@@ -241,9 +244,11 @@ class Interp2Plan:
         return ZI
 
     def scattered(self, XQ, YQ, extrap=np.nan, out=None):
-        """Scattered queries (XQ[k], YQ[k]) -> ZQ[k]."""
-        if _is_torch(XQ):
+        """Scattered queries (XQ[k], YQ[k]) -> ZQ[k].  CUDA tensors run on torch's current stream; numpy arrays take
+        the host path."""
+        if _is_torch(XQ) or _is_torch(YQ):
             import torch
+            _dev_operands(self.dtype, XQ, YQ, *(() if out is None else (out,)))
             ZQ = torch.empty_like(XQ) if out is None else out
             check(_lib.lib().b200_interp2_scattered_dev(self._h, C.c_void_p(XQ.data_ptr()), C.c_void_p(YQ.data_ptr()),
                                                        C.c_size_t(XQ.numel()), C.c_void_p(ZQ.data_ptr()),

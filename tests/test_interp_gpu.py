@@ -120,21 +120,24 @@ def test_interp1_errors(b200):
 
 
 @pytest.mark.parametrize("dt", [np.float64, np.float32])
-def test_interp2_vs_oracle(b200, oracle, dt):
+@pytest.mark.parametrize("y_first", [False, True])
+def test_interp2_vs_oracle(b200, oracle, y_first, dt):
     rng = np.random.default_rng(13)
     nx, ny = 513, 384
     x = np.unique(np.cumsum(0.5 + rng.random(nx)).astype(dt)); y = np.linspace(-2, 3, ny).astype(dt)
     z = rng.standard_normal((y.size, x.size)).astype(dt)
-    plan = b200.Interp2Plan(x, y, z)
+    plan = b200.Interp2Plan(x, y, z, flags=b200.Interp2Plan.ORDER_YX if y_first else 0)
     nq = 300_001
     xq = rng.uniform(x[0] - 1, x[-1] + 1, nq).astype(dt); yq = rng.uniform(-2.1, 3.1, nq).astype(dt)
     xq[:5] = [x[0], x[-1], np.nan, x[3], x[-1]]; yq[:5] = [y[0], y[-1], 0.0, np.nan, y[0]]
     for extrap in (np.nan, 2.25):
-        assert same_bits(plan.scattered(xq, yq, extrap=extrap), oracle.interp2_scattered(x, y, z, xq, yq, extrap=extrap, nthreads=8))
+        assert same_bits(plan.scattered(xq, yq, extrap=extrap),
+                         oracle.interp2_scattered(x, y, z, xq, yq, extrap=extrap, nthreads=8, y_first=y_first))
     xi = rng.uniform(x[0] - 1, x[-1] + 1, 333).astype(dt)
     for nyi in (1000, 1002, 777):                # multiple of 4: 32-byte stores, even: 16-byte, odd: scalar
         yi = rng.uniform(-2.1, 3.1, nyi).astype(dt)
-        assert same_bits(plan.grid(xi, yi, extrap=0.5), oracle.interp2_grid(x, y, z, xi, yi, extrap=0.5, nthreads=8))
+        assert same_bits(plan.grid(xi, yi, extrap=0.5),
+                         oracle.interp2_grid(x, y, z, xi, yi, extrap=0.5, nthreads=8, y_first=y_first))
 
 
 def test_interp2_device_buffers(b200, oracle):
