@@ -11,8 +11,13 @@ GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "interp_golden.
 
 
 def same_bits(a, b):
+    """Equal bits on integer views (so -0.0 and +0.0 differ), NaN compared by position only"""
     a = np.ascontiguousarray(a); b = np.ascontiguousarray(b)
-    return a.shape == b.shape and np.array_equal(np.isnan(a), np.isnan(b)) and np.array_equal(a[~np.isnan(a)], b[~np.isnan(b)])
+    if a.shape != b.shape or a.dtype != b.dtype:
+        return False
+    ints = lambda v: v.view(np.int64 if v.dtype == np.float64 else np.int32)
+    na, nb = np.isnan(a), np.isnan(b)
+    return np.array_equal(na, nb) and np.array_equal(ints(a)[~na], ints(b)[~nb])
 
 
 @pytest.mark.parametrize("tag", ["f64", "f32"])
@@ -400,8 +405,10 @@ def test_branch_free_divide_matches_ieee(b200):
 
 @pytest.mark.parametrize("y_first", [False, True])
 def test_interp2_fast_kernel_special_queries(b200, oracle, y_first):
-    """The straight-line kernel (both axes affine, tile layout, double) hands every query outside its common case
-    to the generic path: out of range in either coordinate, NaN, knot hits, the last row / column, the first bin."""
+    """Host batches on an affine tile plan (double) with the queries the straight-line kernel hands to its slow path:
+    out of range in either coordinate, NaN, knot hits, the last row / column, the first bin.  400 003 queries are one
+    launch below the straight-line kernel's 2^20-query gate, so the generic kernel serves them;
+    tests/test_interp2_scattered.py runs the same kinds of queries through the straight-line kernel itself."""
     rng = np.random.default_rng(41)
     n = 600
     x = np.linspace(-1.0, 2.0, n); y = np.linspace(0.0, 1.0, n + 7)
