@@ -663,7 +663,7 @@ int b200_interp1_adjoint(b200_interp1_plan* p, const void* xi, const void* g, si
   DeviceScope on_plan_device(p->device);
   const size_t esz = p->dtype == B200_F64 ? 8 : 4;
   cudaStream_t st = p->stream[0];
-  return adjoint_host({xi, g}, ni * esz, G, p->ng * esz, need, st,
+  return adjoint_host({{xi, ni * esz}, {g, ni * esz}}, G, p->ng * esz, need, st,
                       [&](const std::vector<void*>& d, void* dG, void* ws) {
                         return b200_interp1_adjoint_dev(p, d[0], d[1], ni, dG, ws, need, st);
                       });

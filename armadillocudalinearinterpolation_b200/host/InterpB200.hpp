@@ -131,6 +131,23 @@ class Interp2Plan {
     ZI.set_size(YI.n_elem, XI.n_elem);
     detail::check(b200_interp2_grid(p_, XI.memptr(), XI.n_elem, YI.memptr(), YI.n_elem, ZI.memptr(), extrapolation_value));
   }
+  // Grid plus the slopes dZ/dX, dZ/dY at every (XI(j), YI(i)), each YI.n_elem x XI.n_elem (rules: b200_interp.h)
+  void GridGrad(const arma::vec& XI, const arma::vec& YI, arma::mat& ZI, arma::mat& DZDX, arma::mat& DZDY,
+                double extrapolation_value = arma::datum::nan) const {
+    ZI.set_size(YI.n_elem, XI.n_elem);
+    DZDX.set_size(YI.n_elem, XI.n_elem);
+    DZDY.set_size(YI.n_elem, XI.n_elem);
+    detail::check(b200_interp2_grid_grad(p_, XI.memptr(), XI.n_elem, YI.memptr(), YI.n_elem, ZI.memptr(), DZDX.memptr(),
+                                         DZDY.memptr(), extrapolation_value));
+  }
+  // dZ = W^T G (Y.n_elem x X.n_elem) with G YI.n_elem x XI.n_elem: the gradient of accu(G % ZI) with respect to Z,
+  // deterministic
+  void GridAdjoint(const arma::vec& XI, const arma::vec& YI, const arma::mat& G, arma::mat& dZ) const {
+    if (G.n_rows != YI.n_elem || G.n_cols != XI.n_elem)
+      throw std::logic_error("b200::Interp2Plan::GridAdjoint: G must be YI.n_elem x XI.n_elem");
+    dZ.set_size(ny_, nx_);
+    detail::check(b200_interp2_grid_adjoint(p_, XI.memptr(), XI.n_elem, YI.memptr(), YI.n_elem, G.memptr(), dZ.memptr()));
+  }
   // (XQ(k), YQ(k)) -> ZQ(k): the per-point restatement of interp2
   void Scattered(const arma::vec& XQ, const arma::vec& YQ, arma::vec& ZQ, double extrapolation_value = arma::datum::nan) const {
     if (XQ.n_elem != YQ.n_elem) throw std::logic_error("b200::Interp2Plan::Scattered: XQ and YQ must have the same number of elements");

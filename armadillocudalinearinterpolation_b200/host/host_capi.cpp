@@ -466,4 +466,45 @@ int b200_host_interp2_scattered_adjoint(const double* x, int nx, const double* y
   } catch (const std::exception& e) { g_err = e.what(); return -1; }
 }
 
+// Interp2Plan(X, Y, Z).GridGrad on XI (nxi) x YI (nyi): zi, dzdx, dzdy column-major nyi x nxi
+int b200_host_interp2_grid_grad(const double* x, int nx, const double* y, int ny, const double* z_colmajor,
+                                const double* xi, int nxi, const double* yi, int nyi, double* zi, double* dzdx,
+                                double* dzdy, double extrap) {
+  try {
+    arma::vec X(nx), Y(ny), XI(nxi), YI(nyi);
+    arma::mat Z(ny, nx), ZI, DX, DY;
+    for (int i = 0; i < nx; ++i) X(i) = x[i];
+    for (int i = 0; i < ny; ++i) Y(i) = y[i];
+    for (int i = 0; i < nx * ny; ++i) Z.memptr()[i] = z_colmajor[i];
+    for (int i = 0; i < nxi; ++i) XI(i) = xi[i];
+    for (int i = 0; i < nyi; ++i) YI(i) = yi[i];
+    b200::Interp2Plan plan(X, Y, Z);
+    plan.GridGrad(XI, YI, ZI, DX, DY, extrap);
+    for (int i = 0; i < nxi * nyi; ++i) { zi[i] = ZI.memptr()[i]; dzdx[i] = DX.memptr()[i]; dzdy[i] = DY.memptr()[i]; }
+    return 0;
+  } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
+// Interp2Plan(X, Y, Z).GridAdjoint with G g_rows x g_cols (column-major): dz (column-major ny x nx); returns -1 with the
+// exception's text when G's shape is not nyi x nxi
+int b200_host_interp2_grid_adjoint(const double* x, int nx, const double* y, int ny, const double* z_colmajor,
+                                   const double* xi, int nxi, const double* yi, int nyi, const double* g, int g_rows,
+                                   int g_cols, double* dz) {
+  try {
+    arma::vec X(nx), Y(ny), XI(nxi), YI(nyi);
+    arma::mat Z(ny, nx), G(g_rows, g_cols), dZ;
+    for (int i = 0; i < nx; ++i) X(i) = x[i];
+    for (int i = 0; i < ny; ++i) Y(i) = y[i];
+    for (int i = 0; i < nx * ny; ++i) Z.memptr()[i] = z_colmajor[i];
+    for (int i = 0; i < nxi; ++i) XI(i) = xi[i];
+    for (int i = 0; i < nyi; ++i) YI(i) = yi[i];
+    for (int i = 0; i < g_rows * g_cols; ++i) G.memptr()[i] = g[i];
+    b200::Interp2Plan plan(X, Y, Z);
+    plan.GridAdjoint(XI, YI, G, dZ);
+    if ((int)dZ.n_rows != ny || (int)dZ.n_cols != nx) { g_err = "dZ has the wrong shape"; return -1; }
+    for (int i = 0; i < nx * ny; ++i) dz[i] = dZ.memptr()[i];
+    return 0;
+  } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
 }  // extern "C"

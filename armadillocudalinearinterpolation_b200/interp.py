@@ -227,10 +227,7 @@ class Interp2Plan:
         on torch's current stream; numpy arrays take the host path."""
         if _is_torch(XI) or _is_torch(YI):
             import torch
-            _dev_operands(self.dtype, XI)
-            _dev_operands(self.dtype, YI)   # checked on its own: XI and YI may differ in length
-            if YI.device != XI.device:
-                raise ValueError("device operands must be on one device")
+            self._grid_axes_dev(XI, YI)
             ZI = torch.empty((XI.numel(), YI.numel()), dtype=XI.dtype, device=XI.device)  # column-major ZI
             check(_lib.lib().b200_interp2_grid_dev(self._h, C.c_void_p(XI.data_ptr()), C.c_size_t(XI.numel()),
                                                   C.c_void_p(YI.data_ptr()), C.c_size_t(YI.numel()),
@@ -242,6 +239,86 @@ class Interp2Plan:
         check(_lib.lib().b200_interp2_grid(self._h, _ptr(XI), C.c_size_t(XI.size), _ptr(YI), C.c_size_t(YI.size),
                                           _ptr(ZI), C.c_double(extrap)))
         return ZI
+
+    def _grid_axes_dev(self, XI, YI):
+        _dev_operands(self.dtype, XI)
+        _dev_operands(self.dtype, YI)   # checked on its own: XI and YI may differ in length
+        if YI.device != XI.device:
+            raise ValueError("device operands must be on one device")
+
+    def grid_grad(self, XI, YI, extrap=np.nan):
+        """Tensor-grid queries with their gradient: returns (ZI, DZDX, DZDY), each of shape (YI.size, XI.size).  ZI has
+        the bits of grid(); the slopes are those scattered_grad gives at every (XI[j], YI[i]) (include/b200_interp.h).
+        CUDA tensors run on torch's current stream and return column-major views; numpy arrays take the host path and
+        return Fortran-ordered arrays."""
+        if _is_torch(XI) or _is_torch(YI):
+            import torch
+            self._grid_axes_dev(XI, YI)
+            out = [torch.empty((XI.numel(), YI.numel()), dtype=XI.dtype, device=XI.device) for _ in range(3)]
+            check(_lib.lib().b200_interp2_grid_grad_dev(self._h, C.c_void_p(XI.data_ptr()), C.c_size_t(XI.numel()),
+                                                       C.c_void_p(YI.data_ptr()), C.c_size_t(YI.numel()),
+                                                       *(C.c_void_p(t.data_ptr()) for t in out), C.c_double(extrap),
+                                                       _torch_stream()))
+            return tuple(t.t() for t in out)
+        XI = _np(XI, self.dtype)
+        YI = _np(YI, self.dtype)
+        out = [np.empty((YI.size, XI.size), self.dtype, order="F") for _ in range(3)]
+        check(_lib.lib().b200_interp2_grid_grad(self._h, _ptr(XI), C.c_size_t(XI.size), _ptr(YI), C.c_size_t(YI.size),
+                                               *(_ptr(a) for a in out), C.c_double(extrap)))
+        return tuple(out)
+
+    def grid_adjoint(self, XI, YI, G):
+        """dZ = W^T G, shape (ny, nx), with G of shape (YI.size, XI.size): the gradient of sum_ij G[i, j] * ZI[i, j] with
+        respect to Z; the bits of scattered_adjoint on the mesh (include/b200_interp.h).  From CUDA tensors: G with
+        strides (1, ld) or (ld, 1) is read in place (anything else is made contiguous), the result is a contiguous
+        (row-major) CUDA tensor written on torch's current stream, and the scratch comes from torch's allocator.  From
+        numpy: a Fortran-ordered array."""
+        if _is_torch(XI) or _is_torch(YI) or _is_torch(G):
+            import torch
+            self._grid_axes_dev(XI, YI)
+            nxi, nyi = XI.numel(), YI.numel()
+            if not (_is_torch(G) and G.is_cuda and G.device == XI.device):
+                raise TypeError("G must be a CUDA tensor on the device of XI and YI")
+            if G.dtype != XI.dtype:
+                raise TypeError(f"G must have the plan's dtype {self.dtype}, not {G.dtype}")
+            if tuple(G.shape) != (nyi, nxi):
+                raise ValueError(f"G must have shape {(nyi, nxi)} (YI.size x XI.size), not {tuple(G.shape)}")
+            s0, s1 = G.stride()
+            if s0 == 1 and s1 >= max(nyi, 1):
+                ldg, g_row_major = s1, 0
+            elif s1 == 1 and s0 >= max(nxi, 1):
+                ldg, g_row_major = s0, 1
+            else:
+                G = G.contiguous()
+                ldg, g_row_major = max(nxi, 1), 1
+            lib = _lib.lib()
+            need = C.c_size_t()
+            check(lib.b200_interp2_grid_adjoint_workspace(self._h, C.c_size_t(nxi), C.c_size_t(nyi), C.byref(need)))
+            ws = torch.empty(max(need.value, 1), dtype=torch.uint8, device=XI.device)
+            dZ = torch.empty((self.ny, self.nx), dtype=XI.dtype, device=XI.device)
+            check(lib.b200_interp2_grid_adjoint_dev(
+                self._h, C.c_void_p(XI.data_ptr()), C.c_size_t(nxi), C.c_void_p(YI.data_ptr()), C.c_size_t(nyi),
+                C.c_void_p(G.data_ptr()), C.c_size_t(ldg), C.c_int(g_row_major), C.c_void_p(dZ.data_ptr()),
+                C.c_size_t(self.nx), C.c_int(1), C.c_void_p(ws.data_ptr()), C.c_size_t(ws.numel()), _torch_stream()))
+            return dZ
+        XI = _np(XI, self.dtype)
+        YI = _np(YI, self.dtype)
+        G = np.asarray(G)
+        if G.shape != (YI.size, XI.size):
+            raise ValueError(f"G must have shape {(YI.size, XI.size)} (YI.size x XI.size), not {G.shape}")
+        Gf = np.asfortranarray(G, dtype=self.dtype)
+        dZ = np.empty((self.ny, self.nx), self.dtype, order="F")
+        check(_lib.lib().b200_interp2_grid_adjoint(self._h, _ptr(XI), C.c_size_t(XI.size), _ptr(YI), C.c_size_t(YI.size),
+                                                  _ptr(Gf), _ptr(dZ)))
+        return dZ
+
+    def grid_torch(self, XI, YI, Z=None, extrap=np.nan):
+        """Differentiable tensor-grid interpolation of CUDA tensors (a torch.autograd.Function): returns ZI of shape
+        (YI.size, XI.size), and gradients flow to XI, YI and Z.  With Z given, the plan first takes Z as its values
+        (set_values, ordered on torch's current stream) and holds them afterwards.  The backward pass uses the slopes
+        saved by the forward pass and grid_adjoint; it never reads the plan's values, so a set_values between forward and
+        backward does not change the gradients.  Once differentiable; no gradient for extrap."""
+        return _grid2_function().apply(XI, YI, Z, self, float(extrap))
 
     def scattered(self, XQ, YQ, extrap=np.nan, out=None):
         """Scattered queries (XQ[k], YQ[k]) -> ZQ[k].  CUDA tensors run on torch's current stream; numpy arrays take
@@ -410,6 +487,45 @@ def _scattered2_function():
 
         _SCATTERED2 = Scattered2
     return _SCATTERED2
+
+
+_GRID2 = None
+
+
+def _grid2_function():
+    """The autograd.Function of Interp2Plan.grid_torch (built on first use: torch is imported only when needed)."""
+    global _GRID2
+    if _GRID2 is None:
+        import torch
+        from torch.autograd.function import once_differentiable
+
+        class Grid2(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, XI, YI, Z, plan, extrap):
+                plan._grid_axes_dev(XI, YI)
+                if Z is not None:
+                    plan.set_values(Z.detach())
+                ctx.plan = plan
+                if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
+                    ZI, DX, DY = plan.grid_grad(XI, YI, extrap)
+                    ctx.save_for_backward(XI, YI, DX, DY)
+                else:
+                    ZI = plan.grid(XI, YI, extrap)
+                    ctx.save_for_backward(XI, YI)
+                return ZI
+
+            @staticmethod
+            @once_differentiable
+            def backward(ctx, g):
+                saved = ctx.saved_tensors
+                XI, YI = saved[0], saved[1]
+                gx = (g * saved[2]).sum(0) if ctx.needs_input_grad[0] else None
+                gy = (g * saved[3]).sum(1) if ctx.needs_input_grad[1] else None
+                gZ = ctx.plan.grid_adjoint(XI, YI, g) if ctx.needs_input_grad[2] else None
+                return gx, gy, gZ, None, None
+
+        _GRID2 = Grid2
+    return _GRID2
 
 
 def interp1(X, Y, XI, extrap=np.nan, return_index=False):

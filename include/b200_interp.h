@@ -214,6 +214,40 @@ int b200_interp2_scattered_adjoint_dev(b200_interp2_plan* plan, const void* xq_d
 int b200_interp2_scattered_adjoint(b200_interp2_plan* plan, const void* xq, const void* yq, const void* g, size_t nq,
                                    void* G);
 
+/* Derivatives of tensor-grid queries.  Take the grid's outputs in column-major order: output (i, j) is query
+ * k = j*nyi + i at (XI[j], YI[i]) — the mesh.  Each rule is the scattered rule above, applied to the mesh.
+ * Gradient: zi has exactly the bits of b200_interp2_grid (in either pass order); dzdx(i,j) and dzdy(i,j) have exactly the
+ * bits b200_interp2_scattered_grad gives for mesh query k: NaN slopes for a NaN coordinate, +0 for any other out-of-range
+ * one, the last cell's slope on the last knot of an axis, the slope of the cell to the right on an interior knot.
+ * zi, dzdx and dzdy are nyi x nxi, column-major.  Empty axes (nxi == 0 or nyi == 0): nothing is written.  The _dev call
+ * uses the plan's scratch for the per-axis brackets, as b200_interp2_grid_dev does: one plan must not run on two streams
+ * at once.  nxi or nyi > 2^31-1 gives B200_ERR_UNSUPPORTED. */
+int b200_interp2_grid_grad(b200_interp2_plan* plan, const void* xi, size_t nxi, const void* yi, size_t nyi, void* zi,
+                           void* dzdx, void* dzdy, double extrap_val);
+int b200_interp2_grid_grad_dev(b200_interp2_plan* plan, const void* xi_dev, size_t nxi, const void* yi_dev, size_t nyi,
+                               void* zi_dev, void* dzdx_dev, void* dzdy_dev, double extrap_val, void* stream);
+/* Adjoint onto the grid: G = W^T g with g an nyi x nxi matrix — the gradient of sum_ij g(i,j)*zi(i,j) with respect to Z.
+ * G has exactly the bits of b200_interp2_scattered_adjoint on the mesh with g[k] = g(k % nyi, k / nyi): the same
+ * (cell key, k, role) order, the same once-rounded terms mul(mul(omx, omy), g), and a zero coefficient still makes a
+ * term (NaN payloads aside: a NaN's payload may come from either operand of an add).  That holds also where nxi*nyi exceeds the scattered call's 2^31-1 limit: the product has no limit here, only
+ * nxi, nyi <= 2^31-1 (else B200_ERR_UNSUPPORTED).  The mesh is never formed and no output is sorted: a stable sort of
+ * each axis by its bracket gives the order of the whole sum, and one pass over the nodes forms every term from the two
+ * axes' weights and g.  Workspace O(nxi + nyi + nx + ny).  The terms of one node are added serially, so a small Z under
+ * a large grid is slow (correct).
+ * g_dev: element (i,j) at j*ldg + i (g_row_major == 0, ldg >= nyi) or i*ldg + j (g_row_major != 0, ldg >= nxi).
+ * G_dev: every G(i,j) written at j*ld + i (row_major == 0, ld >= ny) or i*ld + j (row_major != 0, ld >= nx).
+ * Empty axes give an all-+0 G.  The _dev call uses only the caller's `workspace` of at least the queried size: it
+ * allocates nothing, never synchronises the host and can be captured into a graph.  NULL pointers, a short workspace or
+ * ld / ldg below its minimum give B200_ERR_INVALID_ARG before any device work. */
+int b200_interp2_grid_adjoint_workspace(const b200_interp2_plan* plan, size_t nxi, size_t nyi, size_t* bytes);
+int b200_interp2_grid_adjoint_dev(b200_interp2_plan* plan, const void* xi_dev, size_t nxi, const void* yi_dev, size_t nyi,
+                                  const void* g_dev, size_t ldg, int g_row_major, void* G_dev, size_t ld, int row_major,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+/* Host buffers, g column-major nyi x nxi, G column-major ny x nx (arma::mat): allocates, runs on the plan's internal
+ * stream, synchronous. */
+int b200_interp2_grid_adjoint(b200_interp2_plan* plan, const void* xi, size_t nxi, const void* yi, size_t nyi,
+                              const void* g, void* G);
+
 /* Introspection for the bench: which bracket-lookup path the plan selected
  * (0 = (quasi-)uniform knots: index arithmetic + knot fix-up on one segment record per query,
  *  1 = bucket table + bounded scan / binary search on segment records,
